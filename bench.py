@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- EKF predict+update steps/s at N landmarks, with the covariance sweep's HBM roofline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one whole Robot::localize (slam_ros/Robot.cpp:126-943): prediction, association of the m
 observed lines against every map landmark, the matched updates (folded into one rank-2m covariance
@@ -175,7 +175,7 @@ def cpu_run(workload, steps, warmup, budget_s, threads=None, n_filters=1, extra_
         dt = time.perf_counter() - t0
         fps = done / dt                         # filter-steps per second on one core
         cores = os.cpu_count() or 1
-        return fps / w["filters"], {"kind": "port", "cores": 1, "value": fps / w["filters"], "unit": "steps/s",
+        return fps / w["filters"], {"kind": "port", "cores": 1, "value": fps / w["filters"], "unit": "steps/s", "steps": done,
                                     "all_cores_estimate": {"value": fps * cores / w["filters"], "cores": cores,
                                                            "note": "ESTIMATE: one filter per core, perfect scaling (not measured)"},
                                     "sample": "%d scans of ONE 50-landmark filter on one thread; batch steps/s = filter-steps/s / %d filters (the reference has no threads)" % (done, w["filters"])}
@@ -222,7 +222,7 @@ def cpu_run(workload, steps, warmup, budget_s, threads=None, n_filters=1, extra_
     # + ~0.05 ms per (line, landmark) gate pair; check: the LINESIZE = 1000 build of the reference itself measures 12.7 s
     # per step at n = 2003, m = 8 (bench.py --workload 1k), this formula gives 11.1 s
     lit_ms = 7.1 * (n / 203.0) ** 3 + m * 0.45 * (n / 203.0) ** 2 + m * N * 0.05 * (n / 203.0)
-    info = {"kind": "port", "cores": threads, "value": val, "unit": "steps/s",
+    info = {"kind": "port", "cores": threads, "value": val, "unit": "steps/s", "steps": total_done,
             "literal_reference_extrapolated": "EXTRAPOLATED, not measured: the reference's own dense GSL path would need about "
                                               "%.3g s per step at n = %d (2 n^3 MACs per prediction dgemm)" % (lit_ms / 1e3, n),
             "sample": "%d full steps of the same workload%s on the structured oracle (oracle/ekf_oracle.cpp, the runtime-capacity "
@@ -258,25 +258,33 @@ def literal_1k_run(steps, budget_s):
             break
     dt = time.perf_counter() - t0
     val = done / dt
-    return val, {"kind": "reference", "cores": 1, "value": val, "unit": "steps/s",
+    return val, {"kind": "reference", "cores": 1, "value": val, "unit": "steps/s", "steps": done,
                  "sample": "%d Robot::localize calls of the literal reference compiled with LINESIZE=1000 (n = 2003; g++ -O2, GSL shim, "
                            "cout disabled) on a 980-landmark map, m = 8 -- the structured oracle is bitwise equal to it at this size "
                            "(tests/test_oracle.py)" % done}
 
 
-def literal_run(steps, warmup, budget_s):
-    """configs[0] on the reference ITSELF: oracle/_ref/libslamref.so = slam_ros/Robot.cpp (Q1-patched on a pipe)
-    compiled -O2 over the GSL shim, single thread (the reference has none), std::cout disabled (Q14)."""
-    from oracle.oracle import LiteralReference, have_literal
+def room_cpu_run(steps, warmup, budget_s):
+    """configs[0] on the host: the reference ITSELF where built (oracle/_ref/libslamref.so = slam_ros/Robot.cpp,
+    Q1-patched on a pipe, compiled -O2 over the GSL shim, std::cout disabled (Q14)), else the structured oracle (its
+    bitwise restatement, tests/test_oracle.py); single thread either way (the reference has none)."""
+    from oracle.oracle import LiteralReference, StructuredOracle, have_literal
     from slam_ros_b200 import scenario as sc
-    if not have_literal():
-        return None, {"kind": "reference", "unavailable": "oracle/_ref/libslamref.so not present (built only where /root/reference exists)"}
     room = sc.room_scenario(steps=warmup + steps, seed=7, range_sigma=5e-5)
-    lit = LiteralReference()
-    def step(s):
-        m = room["count"][s]
-        y, P, L, pose = lit.state()
-        lit.localize(room["z"][s, :m], room["R"][s, :m], sc.encoder_for(pose, room["u"][s]))
+    kind = "reference" if have_literal() else "port"
+    if kind == "reference":
+        lit = LiteralReference()
+
+        def step(s):
+            m = room["count"][s]
+            y, P, L, pose = lit.state()
+            lit.localize(room["z"][s, :m], room["R"][s, :m], sc.encoder_for(pose, room["u"][s]))
+    else:
+        so = StructuredOracle(100, threads=1)
+
+        def step(s):
+            m = room["count"][s]
+            so.localize(room["z"][s, :m], room["R"][s, :m], sc.encoder_for(so.pose, room["u"][s]))
     for s in range(warmup):
         step(s)
     t0 = time.perf_counter()
@@ -288,8 +296,11 @@ def literal_run(steps, warmup, budget_s):
             break
     dt = time.perf_counter() - t0
     val = done / dt
-    return val, {"kind": "reference", "cores": 1, "value": val, "unit": "steps/s",
-                 "sample": "%d Robot::localize calls of the literal reference (LINESIZE=100, g++ -O2, GSL shim, cout disabled) on the room scenario, including its state read-back through the harness" % done}
+    what = ("the literal reference (LINESIZE=100, g++ -O2, GSL shim, cout disabled) on the room scenario, including its state "
+            "read-back through the harness") if kind == "reference" else \
+        "the structured oracle (oracle/ekf_oracle.cpp, capacity 100, g++ -O2, one thread) on the room scenario"
+    return val, {"kind": kind, "cores": 1, "value": val, "unit": "steps/s", "steps": done,
+                 "sample": "%d Robot::localize calls of %s" % (done, what)}
 
 
 def run_room(args, rank, world, local):
@@ -350,7 +361,7 @@ def lines_cpu_run(steps, budget_s):
     dt = time.perf_counter() - t0
     what = ("LineExtraction of slam_ros/lineFitting.cpp itself (g++ -O2, GSL shim, zero-initialised locals; it also writes "
             "three text files per call, as in the node)") if kind == "reference" else "oracle/lines_oracle.cpp (g++ -O2)"
-    return done / dt, {"kind": kind, "cores": 1, "value": done / dt, "unit": "scans/s",
+    return done / dt, {"kind": kind, "cores": 1, "value": done / dt, "unit": "scans/s", "steps": done,
                        "sample": "%d scans of the same payloads through %s" % (done, what)}
 
 
@@ -399,14 +410,20 @@ def run_extract(args, rank, world, local):
     }
 
 
+REF_BUDGET_S = 150.0
+
+
 def run_reference_arm(args, rank, world):
+    """`steps` is the number of steps actually timed: the CPU implementations stop after REF_BUDGET_S seconds of
+    timed work, which can be fewer than the --steps requested (`steps_requested`)."""
     if rank != 0:
         return
     w = WORKLOADS[args.workload]
     if args.workload == "extract":
-        val, info = lines_cpu_run(args.steps, budget_s=150.0)
+        val, info = lines_cpu_run(args.steps, budget_s=REF_BUDGET_S)
         print(json.dumps({"impl": "reference", "metric": "line-extraction scans/s (361 beams -> (alfa, r, C_AR, end points) per line)",
-                          "value": val, "unit": "scans/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
+                          "value": val, "unit": "scans/s", "n_gpus": args.gpus, "steps": info["steps"], "steps_requested": args.steps,
+                          "budget_s": REF_BUDGET_S, "warmup": args.warmup,
                           "ms_per_step": 1e3 / val, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64",
                           "data": "synthetic", "config": static_config("extract", args.gpus), "cpu_baseline": info,
                           "e2e": {"value": val, "unit": "scans/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -414,20 +431,18 @@ def run_reference_arm(args, rank, world):
         return
     sharded = args.workload == "40k" and args.gpus > 1
     if args.workload == "1k" and args.lines == 0 and _have_literal_1k():
-        val, info = literal_1k_run(min(args.steps, 8), budget_s=150.0)
+        val, info = literal_1k_run(args.steps, budget_s=REF_BUDGET_S)
     elif args.workload == "room":
-        val, info = literal_run(args.steps, args.warmup, budget_s=150.0)
-        if val is None:
-            print(json.dumps({"impl": "reference", "unavailable": info["unavailable"]}), flush=True)
-            return
+        val, info = room_cpu_run(args.steps, args.warmup, budget_s=REF_BUDGET_S)
     else:
         # replicas at N GPUs = N independent filters: the host runs the same N filters (aggregate rate), so that the
         # driver's ratio compares N GPUs with this one host on the same job
         nf = args.gpus if (args.workload in ("10k", "1k", "40k") and not sharded) else 1
-        val, info = cpu_run(args.workload, args.steps, args.warmup, budget_s=150.0, n_filters=nf)
+        val, info = cpu_run(args.workload, args.steps, args.warmup, budget_s=REF_BUDGET_S, n_filters=nf)
     line = {
         "impl": "reference", "metric": "EKF predict+update steps/s at N landmarks", "value": val, "unit": "steps/s",
-        "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 / val,
+        "n_gpus": args.gpus, "steps": info["steps"], "steps_requested": args.steps, "budget_s": REF_BUDGET_S,
+        "warmup": args.warmup, "ms_per_step": 1e3 / val,
         "higher_is_better": True, "scaling": "strong" if (sharded or (args.workload == "mc" and args.mc_per_gpu == 0)) else "weak",
         "vs_baseline": None, "dtype": "f64", "data": "synthetic",
         "config": static_config(args.workload, args.gpus, sharded, args.mc_per_gpu),
@@ -453,10 +468,38 @@ def _dist_reduce_sum(dev):
     return red
 
 
-def run_filter(wl_name, K, W, rank, world, local, sharded, parity_name=None, exchange_pref="fused", e2e_leg=True):
+DUMP_BLOCKS, DUMP_BLOCK = 64, 32
+
+
+def dump_filter_outputs(f, j_last, out_dir, rank, red):
+    """What a caller of ekf_scan_device holds after the last timed scan, as float64 .npy files in out_dir: that scan's
+    association indices (j.npy, -1 = appended), the pose (pose.npy), the landmark count (lines.npy), the live state
+    vector (y.npy), the robot rows of the covariance (P_robot_rows.npy, 3 x n) and, since P itself is n^2 doubles
+    (3.2 GB at 10k landmarks), DUMP_BLOCKS blocks of DUMP_BLOCK^2 entries of the live covariance: the first and the
+    last diagonal block, the others at seeded origins (P_blocks.npy, with their (row, column) origins in
+    P_block_origins.npy).  A row-sharded filter's ranks all take part (red sums their partial covariance read-outs;
+    y is replicated); rank 0 writes."""
+    pose, L, _ = f.state()
+    nl = 3 + 2 * L
+    y = f.download_y()
+    rows = red(f.download_block(0, 0, 3, nl))
+    b = min(DUMP_BLOCK, nl)
+    origins = np.concatenate([[[0, 0], [nl - b, nl - b]],
+                              np.random.default_rng(12345).integers(0, nl - b + 1, size=(DUMP_BLOCKS - 2, 2))])
+    blocks = np.stack([red(f.download_block(int(r0), int(c0), b, b)) for r0, c0 in origins])
+    if rank != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("j", j_last), ("pose", pose), ("lines", [L]), ("y", y), ("P_robot_rows", rows), ("P_blocks", blocks),
+                    ("P_block_origins", origins)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
+def run_filter(wl_name, K, W, rank, world, local, sharded, parity_name=None, exchange_pref="fused", e2e_leg=True, dump_dir=None):
     """One single-filter workload end to end on this rank's GPU (replica, or this rank's shard of a row-sharded filter).
     parity_name: replay the committed oracle fixture tests/golden/oracle_<name>.npz first (same seeded sequence: the
-    timing legs then continue from where the fixture ends).  Returns a dict of raw measurements (rank 0: complete)."""
+    timing legs then continue from where the fixture ends).  dump_dir: write what the timed leg computed in its last
+    step there (dump_filter_outputs).  Returns a dict of raw measurements (rank 0: complete)."""
     import torch
     import torch.distributed as dist
     from slam_ros_b200 import EkfFilter, scenario as sc
@@ -541,6 +584,9 @@ def run_filter(wl_name, K, W, rank, world, local, sharded, parity_name=None, exc
     f.profile_enable(False)
     matched = int((d_j[W:W + K] >= 0).sum().item())
     pose_dev, L_dev, st_dev = f.state()
+    if dump_dir:
+        dump_filter_outputs(f, d_j[W + K - 1].cpu().numpy(), dump_dir, rank,
+                            _dist_reduce_sum(dev) if shard is not None else (lambda a: a))
 
     # ---- leg 2: end to end through the host-buffer call -------------------------------------------
     e2e_ms, e2e_matched = float("nan"), 0
@@ -600,7 +646,7 @@ def run_single_or_replicas(args, rank, world, local, sharded, wl_name=None, pari
     torch.cuda.set_device(dev)
     if world > 1 and not dist.is_initialized():
         dist.init_process_group("nccl", device_id=dev)
-    r = run_filter(wl_name, K, W, rank, world, local, sharded, parity_name=parity_name)
+    r = run_filter(wl_name, K, W, rank, world, local, sharded, parity_name=parity_name, dump_dir=args.dump_outputs)
     if rank != 0:
         return None
     filters = 1 if sharded else world
@@ -662,7 +708,6 @@ def run_extras(args, rank, world, local):
     # (ii)
     try:
         a = copy.copy(args)
-        a.steps = max(K, 50)
         mc = {}
         a.mc_per_gpu = 0
         ln = run_monte_carlo(a, rank, world, local)
@@ -807,7 +852,14 @@ def main():
                     "un-sharded filter with its parity prefix, Monte-Carlo strong + weak, row-sharded parity on both exchange paths)")
     ap.add_argument("--parity", action="store_true", help="10k / 1k / 40k: replay the committed oracle fixture first and report `parity`")
     ap.add_argument("--cpu-budget", type=float, default=20.0, help="seconds of CPU work for the cpu_baseline sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="10k / 1k / 40k: after the timed steps, write what the timed path "
+                    "computed in its last step to DIR/<name>.npy (float64; the covariance as a seeded sample of blocks); the "
+                    "inputs depend only on the arguments, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in ("10k", "1k", "40k")):
+        ap.error("--dump-outputs needs the GPU arm (--impl ours) of a single-filter workload (10k, 1k, 40k)")
     if args.lines > 0 and args.workload in ("10k", "1k", "40k"):
         w = WORKLOADS[args.workload]
         w["desc"] = w["desc"].replace("m=%d" % w["m"], "m=%d" % args.lines)
@@ -840,7 +892,7 @@ def main():
             if args.workload == "extract":
                 val, info = lines_cpu_run(steps=200, budget_s=args.cpu_budget)
             elif args.workload == "room":
-                val, info = literal_run(steps=1000, warmup=3, budget_s=args.cpu_budget)
+                val, info = room_cpu_run(steps=1000, warmup=3, budget_s=args.cpu_budget)
             elif args.workload == "1k" and args.lines == 0 and _have_literal_1k():
                 val, info = literal_1k_run(steps=2, budget_s=args.cpu_budget)
             else:

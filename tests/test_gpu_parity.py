@@ -278,6 +278,28 @@ def test_robot_mirror_against_literal_reference(libekf):
     assert rel(rb.P_t0, P_l) < TOL and rel(rb.y, y_l) < TOL
 
 
+def test_robot_mirror_against_golden_vectors_of_the_reference(libekf):
+    """The same drive on the outputs the reference's own Robot.cpp produced (tests/golden/room_literal.npz, made by
+    make_golden.py): the fixture's lines and odometry u, savedLineCount and the pose after every step, y and P_t0 where
+    the fixture kept them, the ellipse at the end.  As in the live test, the encoder pose is the one that makes
+    Robot.cpp:140-145 recover u from the mirror's OWN pose: the fixture's encoder poses would turn the last bits in
+    which two poses differ into a difference of odometry (u[2] = theta - encoder[2]), compounding step after step."""
+    from slam_ros_b200 import Robot, Line
+    g = np.load(os.path.join(ROOT, "tests", "golden", "room_literal.npz"))
+    rb = Robot(0, 0, 0)
+    for s in range(g["u"].shape[0]):
+        m = int(g["count"][s])
+        z, R = g["z"][s, :m], g["R"][s, :m]
+        enc = sc.encoder_for((rb.xPos, rb.yPos, rb.thetaPos), g["u"][s])
+        rb.localize([Line(z[i, 0], z[i, 1], R[i]) for i in range(m)], rot=None, encoder=enc)
+        assert rb.savedLineCount == int(g["L"][s]), "step %d" % s
+        assert np.abs(np.array([rb.xPos, rb.yPos, rb.thetaPos]) - g["pose"][s]).max() < 1e-9, "pose at step %d" % s
+        if ("P_%d" % s) in g.files:
+            assert rel(rb.P_t0, g["P_%d" % s]) < TOL and rel(rb.y, g["y_%d" % s]) < TOL, "state at step %d" % s
+    ok, ax, ang = rb.getEllipse()
+    assert ok and np.allclose(ax, g["ellipse"][:2], rtol=1e-5) and abs(ang - g["ellipse"][2]) < 1e-4
+
+
 def test_batch_filters_match_oracle(libekf, oracle_cls):
     from slam_ros_b200 import EkfBatch
     B, N, m, steps = 6, 12, 4, 25
