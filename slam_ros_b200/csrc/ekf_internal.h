@@ -131,10 +131,14 @@ cudaError_t ekf_launch_zero_pending(const EkfGeom& g, const EkfBuffers& b, int m
 int ekf_sweep_grid_ub(const EkfGeom& g, int L_ub);
 
 /* The largest double T with sqrt(T) <= gate (sqrt correctly rounded): Robot.cpp:489's `sqrt(fabs(d2)) > MAHALANOBIS`
- * is then exactly `fabs(d2) > T`. */
+ * is then exactly `fabs(d2) > T`, for every d2 including +-inf and NaN (both forms are false for a NaN d2).
+ *   gate = +inf or NaN: `sqrt(|d2|) > gate` is false for every d2, so T = +inf (nothing is rejected; the search below
+ *                       would never end at +inf, as nextafter(inf, inf) == inf);
+ *   gate < 0:           `sqrt(|d2|) > gate` is true for every non-NaN d2, so T = -1 (everything but NaN is rejected). */
 #include <math.h>
 static inline double ekf_gate_d2max(double gate) {
-  if (!(gate >= 0.0)) return -1.0;                        /* a negative or NaN gate rejects everything / nothing as sqrt would */
+  if (gate != gate || gate == INFINITY) return INFINITY;
+  if (!(gate >= 0.0)) return -1.0;
   double t = gate * gate;
   while (sqrt(t) > gate) t = nextafter(t, 0.0);
   for (;;) { const double u = nextafter(t, INFINITY); if (!(sqrt(u) <= gate)) break; t = u; }

@@ -365,10 +365,18 @@ class EkfBatch:
         self.B = int(n_filters)
         self.capacity = int(capacity_lines)
         self.n = 3 + 2 * self.capacity
+        self._pending = []           # line counts of the submitted, not yet collected steps
 
     def _check(self, rc, where, allow=()):
         if rc != EKF_OK and rc not in allow:
             raise EkfError(rc, where, self._lib.ekf_batch_last_error(self._h).decode())
+        return rc
+
+    def _lines(self, u, z, R):
+        """u (B,3), z (B,m,2), R (B,m,4) as contiguous doubles; m may be 0."""
+        za = _arr(z); Ra = _arr(R)
+        m = za.size // (2 * self.B)
+        return _arr(u, (self.B, 3)), za.reshape(self.B, m, 2), Ra.reshape(self.B, m, 4), m
         return rc
 
     def close(self):
@@ -384,8 +392,7 @@ class EkfBatch:
 
     def scan(self, u, z, R):
         """u (B,3), z (B,m,2), R (B,m,4) -> (status, j_out (B,m), pose (B,3))."""
-        ua = _arr(u, (self.B, 3)); za = _arr(z).reshape(self.B, -1, 2); Ra = _arr(R).reshape(self.B, -1, 4)
-        m = za.shape[1]
+        ua, za, Ra, m = self._lines(u, z, R)
         j = np.full((self.B, max(m, 1)), -1, dtype=np.int32); pose = np.zeros((self.B, 3))
         rc = self._check(self._lib.ekf_batch_scan(self._h, _p(ua), m, _p(za) if m else None, _p(Ra) if m else None,
                                                   j.ctypes.data_as(_ip), _p(pose)), "ekf_batch_scan",
@@ -394,18 +401,17 @@ class EkfBatch:
 
     def submit(self, u, z, R):
         """Pipelined host path: stage one step and return at once (at most two in flight); results come from collect()."""
-        ua = _arr(u, (self.B, 3)); za = _arr(z).reshape(self.B, -1, 2); Ra = _arr(R).reshape(self.B, -1, 4)
-        m = za.shape[1]
+        ua, za, Ra, m = self._lines(u, z, R)
         self._check(self._lib.ekf_batch_submit(self._h, _p(ua), m, _p(za) if m else None, _p(Ra) if m else None), "ekf_batch_submit")
-        self._pending = getattr(self, "_pending", [])
         self._pending.append(m)
 
     def collect(self):
         """(status, j_out (B,m), pose (B,3)) of the OLDEST submitted step."""
-        m = self._pending.pop(0)
+        m = self._pending[0] if self._pending else 0
         j = np.full((self.B, max(m, 1)), -1, dtype=np.int32); pose = np.zeros((self.B, 3))
         rc = self._check(self._lib.ekf_batch_collect(self._h, j.ctypes.data_as(_ip), _p(pose)), "ekf_batch_collect",
                          allow=(EKF_ECAPACITY, EKF_ESINGULAR))
+        self._pending.pop(0)
         return rc, j[:, :m], pose
 
     def scan_device(self, d_u, m, d_z, d_R, d_j_out=0):
