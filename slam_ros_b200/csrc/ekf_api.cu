@@ -97,6 +97,12 @@ struct ekf_ctx {
   int chunk_lines, chunk_above;/* overlapped scans of more than chunk_above lines run as chunks of chunk_lines (EKF_CHUNK, EKF_CHUNK_ABOVE; 0 = never) */
   int slots;                   /* rows of Kp / KSp: max(max_batch, 2 * group) */
   int pg_valid, pg_slot0;
+  /* sweep groups: consecutive overlapped scans whose pending terms share ONE sweep pass (DESIGN section 5).  At most one
+   * group is open; its terms live in half `par` of the slot ring and its sweep is launched when it closes. */
+  int grp_budget;              /* most terms a group may hold (EKF_SWEEP_GROUP; 0 = one sweep per scan) */
+  int grp_open, grp_terms;     /* grp_terms: upper bound of the open group's terms (the sum of its scans' m) */
+  int grp_line_sms;            /* SMs of its scans' line loops (one class per group) */
+  int grp_may_reset;           /* one of its scans may have reset the map */
   EkfScanView* d_view;        /* [2] */
   unsigned long long* d_counters;   /* tile counters of the sweep passes: [0,16) line stream, [16,32) sweep stream */
   cudaEvent_t evE, evF[2];
@@ -182,6 +188,7 @@ int free_line_tables(ekf_ctx* ctx) {
 }
 
 int drain(ekf_ctx* ctx);
+int close_group(ekf_ctx* ctx);
 
 /* (re)allocate everything sized by the number of lines in a scan; only legal between scans */
 int ensure_lines(ekf_ctx* ctx, int m) {
@@ -348,6 +355,7 @@ int enqueue_end(ekf_ctx* ctx, const double* d_z, const double* d_R, int m) {
  * Everything except the overlapped ekf_scan path works on that view. */
 int drain(ekf_ctx* ctx) {
   if (!ctx->overlap) return EKF_OK;
+  { int rc = close_group(ctx); if (rc) return rc; }
   CU(cudaStreamSynchronize(ctx->wstream));
   if (ctx->pg_valid) { ctx->rd ^= 1; ctx->pg_valid = 0; }
   ctx->b.P = ctx->Pbuf[ctx->rd];
@@ -363,11 +371,53 @@ int line_event(ekf_ctx* ctx) {
   return EKF_OK;
 }
 
+/* Hands the pending terms in slot half `par` (nterms: upper bound of their count, snapshot in d_view[par]) to the sweep
+ * stream: the sweep reads the buffer the line stream has been appending to and writes the other one; then the next scan's
+ * line loop reads that source buffer plus these terms, in the other half of the slot ring. */
+int hand_off_sweep(ekf_ctx* ctx, int nterms, int L_ub, int line_sms) {
+  const int par = ctx->par;
+  const int slot0 = par * ctx->group;
+  const int tgt = ctx->pg_valid ? (ctx->rd ^ 1) : ctx->rd;      /* source of this sweep */
+  EkfBuffers bt = ctx->b;
+  bt.P = ctx->Pbuf[tgt];
+  CU(cudaEventRecord(ctx->evE, ctx->stream));
+  CU(cudaStreamWaitEvent(ctx->wstream, ctx->evE, 0));
+  cudaEvent_t e0 = 0, e1 = 0;
+  if (ctx->prof) {
+    if (ctx->ev_used + 2 > ctx->ev.size())
+      for (int i = 0; i < 64; ++i) { cudaEvent_t e; CU(cudaEventCreate(&e)); ctx->ev.push_back(e); }
+    e0 = ctx->ev[ctx->ev_used]; e1 = ctx->ev[ctx->ev_used + 1];
+    CU(cudaEventRecord(e0, ctx->wstream));
+  }
+  CU(ekf_launch_sweep_tma(ctx->g, bt, &ctx->tmap2[tgt], ctx->have_tmap8 ? &ctx->tmap8[tgt] : 0, &ctx->tmapK[0], &ctx->tmapK[1], ctx->Pbuf[tgt ^ 1], slot0, &ctx->d_view[par], ctx->d_counters + 16,
+                          ctx->sweep_shape, nterms, L_ub, ctx->num_sms - line_sms, ctx->wstream,
+                          &ctx->tmap2[tgt ^ 1], ctx->have_tmap8 ? &ctx->tmap8[tgt ^ 1] : 0));
+  { const int per_pass = ekf_sweep_terms_per_pass(ctx->sweep_shape, nterms); ctx->launches += (nterms + per_pass - 1) / per_pass; }
+  if (ctx->prof) {
+    CU(cudaEventRecord(e1, ctx->wstream));
+    ctx->ev_used += 2;
+    ctx->ev_bytes.push_back((double)nterms);
+  }
+  CU(cudaEventRecord(ctx->evF[par], ctx->wstream));
+  ctx->evF_used[par] = 1;
+  ctx->rd = tgt; ctx->pg_valid = 1; ctx->pg_slot0 = slot0;
+  ctx->par ^= 1;
+  ctx->b.P = ctx->Pbuf[ctx->rd];
+  return EKF_OK;
+}
+
+/* launches the sweep of the open group, if any: after it nothing is owed but work already on the streams */
+int close_group(ekf_ctx* ctx) {
+  if (!ctx->grp_open) return EKF_OK;
+  ctx->grp_open = 0;
+  return hand_off_sweep(ctx, ctx->grp_terms, ctx->L_ub, ctx->grp_line_sms);
+}
+
 /* Overlapped form of one Robot::localize (single GPU, m <= group): the line stream runs predict, the
- * line-loop cluster kernel and the end-of-scan kernels against Pbuf[rd] plus the previous scan's still
- * pending terms; the sweep of THIS scan is handed to the sweep stream, where it runs while the next
- * scan's line loop already executes.  Buffers: sweep(s) reads X and writes X^1; the next line loop
- * reads X (complete once sweep(s-1) is done) plus this scan's pending terms. */
+ * line-loop cluster kernel and the end-of-scan kernels against Pbuf[rd] plus the previous group's still
+ * pending terms; the sweep of THIS scan's group is handed to the sweep stream when the group closes, where it
+ * runs while the next group's line loops already execute.  Buffers: sweep(G) reads X and writes X^1; the next
+ * group's line loops read X (complete once sweep(G-1) is done) plus G's pending terms. */
 int enqueue_scan_overlapped(ekf_ctx* ctx, const double* d_u, const double* d_x_t0, int m, const double* d_z, const double* d_R) {
   /* Scans of more than chunk_above (32) lines go through the pipeline as CHUNKS of chunk_lines (16): a chunk's sweep (16 pending terms,
    * one tensor-core pass) runs while the next chunk's line loop executes, exactly as a scan's sweep runs under the next
@@ -375,8 +425,17 @@ int enqueue_scan_overlapped(ekf_ctx* ctx, const double* d_u, const double* d_x_t
    * the sweeps of a 64-line scan hide under its own line loop.  Prediction runs before the first chunk, the end-of-scan
    * kernels after the last; in between k_chunk_mark snapshots the finished chunk for its sweep and restarts the pending
    * list.  Same operations per element in the same order as one line loop + one sweep: identical bits. */
-  const int chunk = (ctx->chunk_lines > 0 && m > ctx->chunk_above && ctx->g.world == 1) ? ctx->chunk_lines : m;
+  const bool chunked = ctx->chunk_lines > 0 && m > ctx->chunk_above && ctx->g.world == 1;
+  const int chunk = chunked ? ctx->chunk_lines : m;
   const int line_sms = line_sms_for(ctx->g.world, ctx->g.cap, m);
+  /* Sweep groups (single GPU, unchunked scans): the scan joins the open group if its terms still fit the budget and its line
+   * loop has the group's width; otherwise the open group is swept first and the scan starts a new one. */
+  const bool groupable = ctx->grp_budget > 0 && !chunked && ctx->g.world == 1;
+  const bool joins = groupable && ctx->grp_open && ctx->grp_terms + m <= ctx->grp_budget && line_sms == ctx->grp_line_sms;
+  if (!joins) { int rc = close_group(ctx); if (rc) return rc; }
+  const int grp_terms = joins ? ctx->grp_terms + m : m;
+  /* the group stays open after this scan if one more scan of the same size would still fit */
+  const bool stays_open = groupable && grp_terms + m <= ctx->grp_budget;
   /* the sweep still in flight was sized to leave last_line_sms SMs free: a wider line loop waits for it (only when the
    * number of lines per scan changes class) */
   if (line_sms > ctx->last_line_sms && ctx->pg_valid && ctx->evF_used[ctx->par ^ 1])
@@ -395,51 +454,44 @@ int enqueue_scan_overlapped(ekf_ctx* ctx, const double* d_u, const double* d_x_t
     const int slot0 = par * ctx->group;
     EkfBuffers b = ctx->b;
     b.P = ctx->Pbuf[ctx->rd];
+    /* a scan that continues the group appends its terms after the group's earlier ones (their count: d_view[par].cnt) */
+    const int* carry = joins ? &ctx->d_view[par].cnt : 0;
     const bool fuse = first && ekf_scan_lines_fuses_predict(ctx->peers_ok ? &ctx->peers : 0) && !ctx->no_fuse;
-    if (first && !fuse) { CU(ekf_launch_predict(ctx->g, b, d_u, d_x_t0, m, ctx->L_ub, ctx->stream)); ctx->launches++; }
+    if (first && !fuse) { CU(ekf_launch_predict(ctx->g, b, d_u, d_x_t0, m, ctx->L_ub, ctx->stream, carry)); ctx->launches++; }
     /* The line loop runs as line_sms cooperative CTAs on the SMs the in-flight sweep leaves free (its
      * persistent grid is num_sms - line_sms): no register / FP64-issue sharing with the sweep. */
     CU(ekf_launch_scan_lines(ctx->g, b, d_z, d_R, line0, line1, line_sms, 1, slot0, ctx->pg_slot0,
                              ctx->pg_valid ? &ctx->d_view[par ^ 1].cnt : 0, ctx->peers_ok ? &ctx->peers : 0, ctx->L_ub, ctx->stream,
-                             fuse ? d_u : 0, fuse ? d_x_t0 : 0, m));
+                             fuse ? d_u : 0, fuse ? d_x_t0 : 0, m, fuse ? carry : 0));
     ctx->launches++;
-    const int tgt = ctx->pg_valid ? (ctx->rd ^ 1) : ctx->rd;      /* source of this chunk's sweep */
+    const int tgt = ctx->pg_valid ? (ctx->rd ^ 1) : ctx->rd;      /* source of the next sweep */
     EkfBuffers bt = ctx->b;
     bt.P = ctx->Pbuf[tgt];
     if (last) {
-      CU(ekf_launch_end_scan(ctx->g, bt, d_z, d_R, m, ctx->L_ub, slot0, &ctx->d_view[par], ctx->stream));
+      /* After a map reset earlier in the group, the new landmarks reuse rows and columns that are live for the sweep still
+       * in flight (it writes Pbuf[tgt] and reads Pbuf[rd] there): the end of this scan waits for that sweep. */
+      if (joins && ctx->grp_may_reset && ctx->pg_valid && ctx->evF_used[par ^ 1])
+        CU(cudaStreamWaitEvent(ctx->stream, ctx->evF[par ^ 1], 0));
+      /* while the group stays open, the next scan reads Pbuf[rd] (not the sweep's source) and corrects against the previous
+       * group's terms at every landmark, the new ones included */
+      const bool keep = stays_open && tgt != ctx->rd;
+      CU(ekf_launch_end_scan(ctx->g, bt, d_z, d_R, m, ctx->L_ub, slot0, &ctx->d_view[par], ctx->stream,
+                             keep ? ctx->Pbuf[ctx->rd] : 0, ctx->pg_slot0, (stays_open && ctx->pg_valid) ? &ctx->d_view[par ^ 1].cnt : 0));
       ctx->launches += 2;
       int rc = line_event(ctx); if (rc) return rc;
     } else {
       CU(ekf_launch_chunk_mark(ctx->b, line1, &ctx->d_view[par], ctx->stream));
       ctx->launches++;
     }
-    CU(cudaEventRecord(ctx->evE, ctx->stream));
-    CU(cudaStreamWaitEvent(ctx->wstream, ctx->evE, 0));
-    cudaEvent_t e0 = 0, e1 = 0;
-    if (ctx->prof) {
-      if (ctx->ev_used + 2 > ctx->ev.size())
-        for (int i = 0; i < 64; ++i) { cudaEvent_t e; CU(cudaEventCreate(&e)); ctx->ev.push_back(e); }
-      e0 = ctx->ev[ctx->ev_used]; e1 = ctx->ev[ctx->ev_used + 1];
-      CU(cudaEventRecord(e0, ctx->wstream));
-    }
-    const int nterms = line1 - line0;
-    CU(ekf_launch_sweep_tma(ctx->g, bt, &ctx->tmap2[tgt], ctx->have_tmap8 ? &ctx->tmap8[tgt] : 0, &ctx->tmapK[0], &ctx->tmapK[1], ctx->Pbuf[tgt ^ 1], slot0, &ctx->d_view[par], ctx->d_counters + 16,
-                            ctx->sweep_shape, nterms, L_after_ub, ctx->num_sms - line_sms, ctx->wstream,
-                            &ctx->tmap2[tgt ^ 1], ctx->have_tmap8 ? &ctx->tmap8[tgt ^ 1] : 0));
-    { const int per_pass = ekf_sweep_terms_per_pass(ctx->sweep_shape, nterms); ctx->launches += (nterms + per_pass - 1) / per_pass; }
-    if (ctx->prof) {
-      CU(cudaEventRecord(e1, ctx->wstream));
-      ctx->ev_used += 2;
-      ctx->ev_bytes.push_back((double)nterms);
-    }
-    CU(cudaEventRecord(ctx->evF[par], ctx->wstream));
-    ctx->evF_used[par] = 1;
-    ctx->rd = tgt; ctx->pg_valid = 1; ctx->pg_slot0 = slot0;
-    ctx->par ^= 1;
+    if (!groupable) { int rc = hand_off_sweep(ctx, line1 - line0, L_after_ub, line_sms); if (rc) return rc; }
+  }
+  if (groupable) {
+    ctx->grp_may_reset = (joins && ctx->grp_may_reset) || (long long)ctx->L_ub + m > (long long)ctx->g.cap - ctx->g.headroom;
+    ctx->grp_open = 1; ctx->grp_terms = grp_terms; ctx->grp_line_sms = line_sms;
   }
   ctx->L_ub = L_after_ub;
   ctx->b.P = ctx->Pbuf[ctx->rd];
+  if (ctx->grp_open && !stays_open) return close_group(ctx);
   return EKF_OK;
 }
 
@@ -589,7 +641,8 @@ int create_common(ekf_ctx** out, const ekf_config* cfg, int rank, int world, con
   { const char* e = getenv("EKF_CHUNK"); ctx->chunk_lines = e ? atoi(e) : 16; if (ctx->chunk_lines < 0) ctx->chunk_lines = 0; }
   { const char* e = getenv("EKF_FUSE_PREDICT"); ctx->no_fuse = (e && atoi(e) == 0) ? 1 : 0; }
   { const char* e = getenv("EKF_CHUNK_ABOVE"); ctx->chunk_above = e ? atoi(e) : 32; if (ctx->chunk_above < 1) ctx->chunk_above = 1; }
-  ctx->pg_valid = 0; ctx->pg_slot0 = 0; ctx->d_view = 0; ctx->d_counters = 0; ctx->evE = 0; ctx->evF[0] = ctx->evF[1] = 0;
+  ctx->pg_valid = 0; ctx->pg_slot0 = 0; ctx->d_view = 0;
+  ctx->grp_open = 0; ctx->grp_terms = 0; ctx->grp_line_sms = 0; ctx->grp_may_reset = 0; ctx->d_counters = 0; ctx->evE = 0; ctx->evF[0] = ctx->evF[1] = 0;
   ctx->evF_used[0] = ctx->evF_used[1] = 0; memset(ctx->tab, 0, sizeof ctx->tab);
   ctx->last_line_sms = 64; ctx->arena = 0; ctx->arena_bytes = 0; ctx->h_snap = 0; ctx->ev_snap = 0; ctx->snap_inflight = 0; ctx->snap_added = 0; ctx->xchg = 0; ctx->poisoned = 0; ctx->peers_ok = 0; ctx->peers_mapped = 0; memset(ctx->peer_map, 0, sizeof ctx->peer_map); memset(&ctx->peers, 0, sizeof ctx->peers);
   *out = ctx;                                  /* so the caller can read ekf_last_error on failure */
@@ -647,6 +700,12 @@ int create_common(ekf_ctx** out, const ekf_config* cfg, int rank, int world, con
   { const char* e = getenv("EKF_SWEEP_SHAPE"); ctx->sweep_shape = e ? atoi(e) : 0; if (ctx->sweep_shape < 0 || (ctx->sweep_shape > 5 && ctx->sweep_shape != 8 && ctx->sweep_shape != 9 && ctx->sweep_shape != 10 && ctx->sweep_shape != 11) || ctx->sweep_shape == 3) ctx->sweep_shape = 0; }
   { const int cap = 2 * ekf_sweep_terms_per_pass(ctx->sweep_shape, 64); if (ctx->group > cap) ctx->group = cap; if (ctx->group < 1) ctx->group = 1; }
   if (ctx->chunk_lines > ctx->group) ctx->chunk_lines = ctx->group;          /* a chunk's terms live in one half of the slot ring */
+  /* Terms per sweep group: 16, the largest pass that is still HBM-bound at 10k landmarks (DESIGN section 4.1: 0.504 ms
+   * against 0.491 for 8 terms).  A group's terms live in one half of the slot ring, and a line corrects against the previous
+   * group's terms plus its own group's: both fit the ring half (group) and FL_MAXP (128 >= 2 x group). */
+  { const char* e = getenv("EKF_SWEEP_GROUP"); ctx->grp_budget = e ? atoi(e) : 16; }
+  if (ctx->grp_budget < 0) ctx->grp_budget = 0;
+  if (ctx->grp_budget > ctx->group) ctx->grp_budget = ctx->group;
   { int rc = make_tensor_map(ctx, p_rows, ctx->Pbuf[0], &ctx->tmap2[0]); if (rc) return rc; }
   ctx->have_tmap8 = (ctx->sweep_shape == 0 || ctx->sweep_shape == 10);
   if (ctx->have_tmap8) { int rc = make_tensor_map(ctx, p_rows, ctx->Pbuf[0], &ctx->tmap8[0], 10); if (rc) return rc; }
@@ -895,6 +954,7 @@ int ekf_scan_device(ekf_ctx* ctx, const double* d_u, int m, const double* d_z, c
 int ekf_sync(ekf_ctx* ctx) {
   if (!ctx) return EKF_EINVAL;
   CU(cudaSetDevice(ctx->cfg.device));
+  { int rc = close_group(ctx); if (rc) return rc; }   /* returns with no work owed: the open sweep group is swept too */
   CU(cudaStreamSynchronize(ctx->stream));
   if (ctx->wstream) CU(cudaStreamSynchronize(ctx->wstream));
   return EKF_OK;
@@ -1232,7 +1292,8 @@ int ekf_timer_start(ekf_ctx* ctx) {
 int ekf_timer_stop(ekf_ctx* ctx, double* ms) {
   if (!ctx || !ctx->t0) return EKF_EINVAL;
   CU(cudaSetDevice(ctx->cfg.device));
-  if (ctx->overlap) {          /* the sweeps in flight belong to the timed work */
+  if (ctx->overlap) {          /* the sweeps in flight belong to the timed work, and so does the sweep of the open group */
+    { int rc = close_group(ctx); if (rc) return rc; }
     for (int p = 0; p < 2; ++p) if (ctx->evF_used[p]) CU(cudaStreamWaitEvent(ctx->stream, ctx->evF[p], 0));
   }
   CU(cudaEventRecord(ctx->t1, ctx->stream));

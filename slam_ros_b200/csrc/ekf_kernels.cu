@@ -74,9 +74,12 @@ __global__ void k_init(EkfGeom g, EkfBuffers b) {
 
 /* Robot.cpp:130-258 (structured: SURVEY appendix A.2).  Also opens the scan: per-line tables. */
 /* Robot.cpp:130-258 (+ the per-scan resets of :294) for thread gid of stride: the body of k_predict, also run as the
- * prologue of the one-barrier line loop (k_scan_lines2 with u != NULL: one launch less on the latency path of small maps) */
+ * prologue of the one-barrier line loop (k_scan_lines2 with u != NULL: one launch less on the latency path of small maps).
+ * carry != NULL: the scan continues a sweep group (DESIGN section 5) whose earlier scans left *carry pending terms; its own
+ * terms are appended after them (pbase = -*carry), so the group's one sweep folds them all in order. */
 __device__ __forceinline__ void predict_body(const EkfGeom& g, const EkfBuffers& b, const double* __restrict__ u,
-                                             const double* __restrict__ x_t0, int m, int gid, int stride) {
+                                             const double* __restrict__ x_t0, int m, int gid, int stride,
+                                             const int* __restrict__ carry) {
   EkfDevState* st = b.st;
   const double* x = x_t0 ? x_t0 : st->pose;
   const double x0 = x[0], x1 = x[1], x2 = x[2];
@@ -141,13 +144,13 @@ __device__ __forceinline__ void predict_body(const EkfGeom& g, const EkfBuffers&
     st->x_pre[2] = add_rn(x2, u2);
     if (x_t0) { st->pose[0] = x0; st->pose[1] = x1; st->pose[2] = x2; }
     st->epoch += 1;                                                   /* matchSavedIndexes.clear(), :294 */
-    st->pbase = 0; st->np = 0;
+    st->pbase = carry ? -*carry : 0; st->np = 0;
     b.pidx[0] = 0; b.eidx[0] = 0;
   }
 }
 __global__ void __launch_bounds__(EKF_BLOCK) k_predict(EkfGeom g, EkfBuffers b, const double* __restrict__ u,
-                                                       const double* __restrict__ x_t0, int m) {
-  predict_body(g, b, u, x_t0, m, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
+                                                       const double* __restrict__ x_t0, int m, const int* __restrict__ carry) {
+  predict_body(g, b, u, x_t0, m, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x, carry);
 }
 
 /* Robot.cpp:313-501 for one line: every un-matched landmark is gated in parallel; first fit = the
@@ -720,7 +723,8 @@ template <int FL_THREADS, bool COOP, bool CACHED>
 __global__ void __launch_bounds__(FL_THREADS, 1) k_scan_lines2(EkfGeom g, EkfBuffers b, const double* __restrict__ z,
                                                                const double* __restrict__ R, int line0, int line1,
                                                                int own_slot0, int prev_slot0, const int* __restrict__ prev_cnt_ptr,
-                                                               const double* __restrict__ pred_u, const double* __restrict__ pred_x, int pred_m) {
+                                                               const double* __restrict__ pred_u, const double* __restrict__ pred_x, int pred_m,
+                                                               const int* __restrict__ pred_carry) {
   __shared__ int s_min[FL_THREADS / 32];
   __shared__ double2 s_ka[FL_MAXP], s_kb[FL_MAXP], s_ksa[FL_MAXP], s_ksb[FL_MAXP];
   const int prev_cnt = prev_cnt_ptr ? *prev_cnt_ptr : 0;   /* previous scan's terms not yet folded into b.P */
@@ -732,7 +736,7 @@ __global__ void __launch_bounds__(FL_THREADS, 1) k_scan_lines2(EkfGeom g, EkfBuf
     if (COOP) cg::this_grid().sync(); else cg::this_cluster().sync();
   };
   if (pred_u) {                        /* the scan's prediction as the prologue of its (first) line-loop launch */
-    predict_body(g, b, pred_u, pred_x, pred_m, gtid, gstride);
+    predict_body(g, b, pred_u, pred_x, pred_m, gtid, gstride, pred_carry);
     __threadfence();
     group_sync();
   }
@@ -1537,7 +1541,7 @@ k_sweep_dmma(EkfGeom g, EkfBuffers b, const __grid_constant__ CUtensorMap tmapP,
 /* Robot.cpp:702-716 then :776-866 phase A (per unmatched line: world-frame parameters, P_ll, and the
  * rows 0..2 of its new columns -- all functions of the 3x3 robot block only). */
 __global__ void __launch_bounds__(512) k_end_scan_a(EkfGeom g, EkfBuffers b, const double* __restrict__ z, const double* __restrict__ R, int m,
-                                                    int slot0, EkfScanView* view) {
+                                                    int slot0, EkfScanView* view, int prev_slot0, const int* __restrict__ prev_cnt_ptr) {
   EkfDevState* st = b.st;
   __shared__ double s_pose[3];
   __shared__ double s_y01[2];
@@ -1561,13 +1565,18 @@ __global__ void __launch_bounds__(512) k_end_scan_a(EkfGeom g, EkfBuffers b, con
   }
   /* this scan's pending terms have no entry for the rows being appended: zero them, so that the (possibly
    * later) sweep and the next scan's on-the-fly corrections see K = 0 there */
+  /* prev_cnt_ptr != NULL (a sweep group stays open): the same for the terms of the previous group, which the group's next
+   * scan still corrects against -- a term contributes exactly zero at every row appended after it was formed */
   {
     const int cnt = b.pidx[m] - st->pbase, r0 = 3 + 2 * L, r1 = 3 + 2 * (L + n_add);
-    for (int i = 0; i < cnt; ++i)
+    const int pcnt = prev_cnt_ptr ? *prev_cnt_ptr : 0;
+    for (int i = 0; i < cnt + pcnt; ++i) {
+      const size_t slot = i < cnt ? slot0 + i : prev_slot0 + (i - cnt);
       for (int r = r0 + threadIdx.x; r < r1; r += blockDim.x) {
-        b.Kp[(size_t)(slot0 + i) * g.ld + r] = make_double2(0.0, 0.0);
-        b.KSp[(size_t)(slot0 + i) * g.ld + r] = make_double2(0.0, 0.0);
+        b.Kp[slot * g.ld + r] = make_double2(0.0, 0.0);
+        b.KSp[slot * g.ld + r] = make_double2(0.0, 0.0);
       }
+    }
   }
   double A[3][3];
   load_rr(g, b.top, A);
@@ -1628,15 +1637,20 @@ __global__ void __launch_bounds__(512) k_end_scan_a(EkfGeom g, EkfBuffers b, con
   if (threadIdx.x == 0) {
     st->L0 = L;
     int Ln = L + n_add;
-    if (Ln > g.cap - g.headroom) { Ln = 0; st->resets += 1; }
+    const bool reset = Ln > g.cap - g.headroom;
+    if (reset) { Ln = 0; st->resets += 1; }
     st->L = Ln;
-    if (view) { view->cnt = b.pidx[m] - st->pbase; view->L = Ln; }   /* what this scan's sweep will need */
+    /* what this scan's sweep will need.  A reset voids the pending terms (they describe the old map): a scan that continues
+     * the sweep group carries none of them, and the group's sweep folds only terms formed after the reset. */
+    if (view) { view->cnt = reset ? 0 : b.pidx[m] - st->pbase; view->L = Ln; }
   }
 }
 
 /* Robot.cpp:856-860 phase B: the new landmarks' column blocks P[k, l..l+1] = Gx * P[0:3, k], 3 <= k < l.
  * Threads run along the new columns (coalesced row writes); blockIdx.y strides over the rows. */
-__global__ void __launch_bounds__(EKF_BLOCK) k_end_scan_b(EkfGeom g, EkfBuffers b) {
+/* P2 != NULL: the new columns go into that buffer too -- the covariance the next scan of an open sweep group reads
+ * (DESIGN section 5); there they are dead columns of the sweep in flight, which reads that buffer. */
+__global__ void __launch_bounds__(EKF_BLOCK) k_end_scan_b(EkfGeom g, EkfBuffers b, double* __restrict__ P2) {
   const EkfDevState* st = b.st;
   const int n_add = st->n_added;
   const int L = st->L0;                                        /* lines before this scan's append (k_end_scan_a) */
@@ -1653,6 +1667,7 @@ __global__ void __launch_bounds__(EKF_BLOCK) k_end_scan_b(EkfGeom g, EkfBuffers 
     if (tsel == 0) { v = 0.0; axpy_skip(v, 1.0, t2p[k]); }
     else { v = 0.0; axpy_skip(v, cw, t0p[k]); axpy_skip(v, sw, t1p[k]); }
     b.P[local_row(g, k) * g.ld + col] = v;
+    if (P2) P2[local_row(g, k) * g.ld + col] = v;
   }
 }
 
@@ -1755,9 +1770,9 @@ cudaError_t ekf_launch_init(const EkfGeom& g, const EkfBuffers& b, cudaStream_t 
   return cudaGetLastError();
 }
 cudaError_t ekf_launch_predict(const EkfGeom& g, const EkfBuffers& b, const double* d_u, const double* d_x_t0,
-                               int m, int L_ub, cudaStream_t s) {
+                               int m, int L_ub, cudaStream_t s, const int* carry) {
   const int work = (3 + 2 * L_ub > m) ? 3 + 2 * L_ub : m;
-  k_predict<<<blocks_for(work, 1024), EKF_BLOCK, 0, s>>>(g, b, d_u, d_x_t0, m);
+  k_predict<<<blocks_for(work, 1024), EKF_BLOCK, 0, s>>>(g, b, d_u, d_x_t0, m, carry);
   return cudaGetLastError();
 }
 cudaError_t ekf_launch_associate(const EkfGeom& g, const EkfBuffers& b, const double* d_z, const double* d_R,
@@ -1832,7 +1847,7 @@ int ekf_scan_lines_fuses_predict(const EkfPeers* peers) { return !line_loop_v1()
 cudaError_t ekf_launch_scan_lines(const EkfGeom& g, const EkfBuffers& b, const double* d_z, const double* d_R,
                                   int line0, int line1, int ctas, int coop, int own_slot0, int prev_slot0,
                                   const int* prev_cnt_ptr, const EkfPeers* peers, int L_ub, cudaStream_t s,
-                                  const double* pred_u, const double* pred_x, int pred_m) {
+                                  const double* pred_u, const double* pred_x, int pred_m, const int* pred_carry) {
   if (line1 <= line0) return cudaSuccess;
   if (pred_u && !ekf_scan_lines_fuses_predict(peers)) return cudaErrorInvalidValue;
   EkfPeers pe;
@@ -1847,7 +1862,7 @@ cudaError_t ekf_launch_scan_lines(const EkfGeom& g, const EkfBuffers& b, const d
     if (line_loop_v1())
       return cudaLaunchCooperativeKernel((const void*)k_scan_lines<512, true, false>, dim3(ctas), dim3(512), args, 0, s);
     void* args2[] = {(void*)&g, (void*)&b, (void*)&d_z, (void*)&d_R, (void*)&line0, (void*)&line1, (void*)&own_slot0,
-                     (void*)&prev_slot0, (void*)&prev_cnt_ptr, (void*)&pred_u, (void*)&pred_x, (void*)&pred_m};
+                     (void*)&prev_slot0, (void*)&prev_cnt_ptr, (void*)&pred_u, (void*)&pred_x, (void*)&pred_m, (void*)&pred_carry};
     /* 256-thread CTAs (EKF_LINE_THREADS=256, twice the SMs for the same map): up to 255 registers per thread -- none of the
      * line loop's state spills */
     static int lt = -1;
@@ -1871,11 +1886,11 @@ cudaError_t ekf_launch_scan_lines(const EkfGeom& g, const EkfBuffers& b, const d
   if (L_ub <= ctas * 256) {
     /* small maps: 256-thread CTAs may use up to 255 registers -- no spills on the per-line critical path */
     cfg.blockDim = dim3(256);
-    return cudaLaunchKernelEx(&cfg, k_scan_lines2<256, false, true>, g, b, d_z, d_R, line0, line1, own_slot0, prev_slot0, prev_cnt_ptr, pred_u, pred_x, pred_m);
+    return cudaLaunchKernelEx(&cfg, k_scan_lines2<256, false, true>, g, b, d_z, d_R, line0, line1, own_slot0, prev_slot0, prev_cnt_ptr, pred_u, pred_x, pred_m, pred_carry);
   }
   if (L_ub <= ctas * 512)
-    return cudaLaunchKernelEx(&cfg, k_scan_lines2<512, false, true>, g, b, d_z, d_R, line0, line1, own_slot0, prev_slot0, prev_cnt_ptr, pred_u, pred_x, pred_m);
-  return cudaLaunchKernelEx(&cfg, k_scan_lines2<512, false, false>, g, b, d_z, d_R, line0, line1, own_slot0, prev_slot0, prev_cnt_ptr, pred_u, pred_x, pred_m);
+    return cudaLaunchKernelEx(&cfg, k_scan_lines2<512, false, true>, g, b, d_z, d_R, line0, line1, own_slot0, prev_slot0, prev_cnt_ptr, pred_u, pred_x, pred_m, pred_carry);
+  return cudaLaunchKernelEx(&cfg, k_scan_lines2<512, false, false>, g, b, d_z, d_R, line0, line1, own_slot0, prev_slot0, prev_cnt_ptr, pred_u, pred_x, pred_m, pred_carry);
 }
 cudaError_t ekf_launch_flush_done(const EkfBuffers& b, int next_line, cudaStream_t s) {
   k_flush_done<<<1, 32, 0, s>>>(b, next_line);
@@ -2068,10 +2083,11 @@ cudaError_t ekf_launch_sweep_tma(const EkfGeom& g, const EkfBuffers& b, const vo
   }
 }
 cudaError_t ekf_launch_end_scan(const EkfGeom& g, const EkfBuffers& b, const double* d_z, const double* d_R,
-                                int m, int L_ub, int slot0, EkfScanView* view, cudaStream_t s) {
+                                int m, int L_ub, int slot0, EkfScanView* view, cudaStream_t s,
+                                double* P2, int prev_slot0, const int* prev_cnt_ptr) {
   /* all blocks of phase A redo the (idempotent) no-match bookkeeping only in thread 0 of block 0's
    * shared copy; to keep it race-free phase A runs as ONE block when it also has to write the pose */
-  k_end_scan_a<<<1, 512, 0, s>>>(g, b, d_z, d_R, m, slot0, view);
+  k_end_scan_a<<<1, 512, 0, s>>>(g, b, d_z, d_R, m, slot0, view, prev_slot0, prev_cnt_ptr);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return e;
   if (m > 0) {
@@ -2080,7 +2096,7 @@ cudaError_t ekf_launch_end_scan(const EkfGeom& g, const EkfBuffers& b, const dou
     if (rows_ub > g.n) rows_ub = g.n;
     int gy = rows_ub / 8; if (gy < 1) gy = 1; if (gy > 2048) gy = 2048;
     dim3 grid((cols_ub + EKF_BLOCK - 1) / EKF_BLOCK, gy);
-    k_end_scan_b<<<grid, EKF_BLOCK, 0, s>>>(g, b);
+    k_end_scan_b<<<grid, EKF_BLOCK, 0, s>>>(g, b, P2);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
   }
