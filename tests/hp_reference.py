@@ -106,14 +106,27 @@ class HPFilter:
         self.my = np.zeros(n); self.my[:nl] = _f(self.y[:nl])
         self.pose = self.y[:3].copy(); self.mpose = self.my[:3].copy()
         self.xp = self.pose.copy(); self.mxp = self.mpose.copy()
-        P = np.asarray(P, np.float64)
-        self.base = np.zeros((n, n)); self.base[:nl, :nl] = P[:nl, :nl]
+        # only the live nl x nl part is kept (entries outside it read as zero; appended rows come from `aug`), so a
+        # filter of large capacity costs memory in proportion to its uploaded map, not to n^2
+        self.base = np.array(np.asarray(P, np.float64)[:nl, :nl])
         self.T = np.zeros((3, n), LD); self.T[:, :nl] = self.base[:3, :nl]
         self.mT = _f(self.T)
         self.aug = {}                # appended row -> (values over columns <= its pair, magnitudes)
-        self.K = []; self.KS = []; self.mK = []; self.mKS = []
-        self._cat = None
+        self._clear_terms()
         self.depth = DEPTH_GAIN
+
+    def _clear_terms(self):
+        self.nt = 0                  # number of pending-term columns (2 per matched line) in the buffers below
+        self._tb = [np.zeros((self.n, 0), LD), np.zeros((self.n, 0), LD), np.zeros((self.n, 0)), np.zeros((self.n, 0))]
+
+    def _base(self, r, c):
+        """base[r][:, c] (index arrays), zero outside the uploaded live block."""
+        nb = self.base.shape[0]
+        out = np.zeros((r.size, c.size))
+        ri = np.nonzero(r < nb)[0]; ci = np.nonzero(c < nb)[0]
+        if ri.size and ci.size:
+            out[np.ix_(ri, ci)] = self.base[np.ix_(r[ri], c[ci])]
+        return out
 
     @property
     def C(self):
@@ -124,19 +137,25 @@ class HPFilter:
         return 3 + 2 * self.L
 
     def _terms(self):
-        if self._cat is None:
-            n = self.n
-            if self.K:
-                self._cat = (np.concatenate(self.K, 1), np.concatenate(self.KS, 1),
-                             np.concatenate(self.mK, 1), np.concatenate(self.mKS, 1))
-            else:
-                self._cat = (np.zeros((n, 0), LD), np.zeros((n, 0), LD), np.zeros((n, 0)), np.zeros((n, 0)))
-        return self._cat
+        """(K, KS, mag K, mag KS), n x 2k: the k pending terms in the order they were formed."""
+        return tuple(b[:, :self.nt] for b in self._tb)
+
+    def _add_term(self, K, KS, mK, mKS):
+        if self.nt + 2 > self._tb[0].shape[1]:           # grow geometrically: appending stays O(n) per term
+            w = max(16, 2 * self._tb[0].shape[1])
+            grown = []
+            for b in self._tb:
+                g = np.zeros((self.n, w), b.dtype); g[:, :self.nt] = b[:, :self.nt]
+                grown.append(g)
+            self._tb = grown
+        for b, v in zip(self._tb, (K, KS, mK, mKS)):
+            b[:, self.nt:self.nt + 2] = v
+        self.nt += 2
 
     def block(self, rows, cols):
         """(value, magnitude) of P[rows][:, cols] (index arrays or ranges)."""
         r = np.asarray(rows, dtype=np.int64).reshape(-1); c = np.asarray(cols, dtype=np.int64).reshape(-1)
-        val = self.base[np.ix_(r, c)].astype(LD)
+        val = self._base(r, c).astype(LD)
         for l, (v, mv) in sorted(self.aug.items()):
             ri = np.nonzero(r == l)[0]; ci = np.nonzero(c == l)[0]
             if ri.size:
@@ -176,7 +195,9 @@ class HPFilter:
         a = 3 + 2 * np.asarray(js, np.int64); b = a + 1
         out = []
         for p, q in ((a, a), (a, b), (b, b)):
-            v = self.base[p, q].astype(LD); m = _f(v)
+            nb = self.base.shape[0]
+            inb = (p < nb) & (q < nb)
+            v = np.zeros(p.size, LD); v[inb] = self.base[p[inb], q[inb]]; m = _f(v)
             hi = np.maximum(p, q); lo = np.minimum(p, q)
             for key, (av, am) in self.aug.items():
                 i = np.nonzero(hi == key)[0]
@@ -301,7 +322,7 @@ class HPFilter:
         # rows 0-2 explicitly, the rest through the term list
         self.T = self.T - KS[:3] @ K.T
         self.mT = self.mT + mKS[:3] @ mK.T
-        self.K.append(K); self.KS.append(KS); self.mK.append(mK); self.mKS.append(mKS); self._cat = None
+        self._add_term(K, KS, mK, mKS)
         self.y[:3] = self.xp; self.my[:3] = self.mxp
         self.y = self.y + K @ v
         self.my = self.my + mK @ _f(v) + _f(K) @ mv
@@ -367,12 +388,11 @@ class HPFilter:
                 break
             self._augment(z[i], R[i])
         if self.L > self.cap - self.headroom:                          # Robot.cpp:893-904
-            n = self.n
             self.L = 0
             self.y[3:] = 0; self.my[3:] = 0
             self.T[:, 3:] = 0; self.mT[:, 3:] = 0
-            self.base = np.zeros((n, n)); self.aug = {}
-            self.K = []; self.KS = []; self.mK = []; self.mKS = []; self._cat = None
+            self.base = np.zeros((0, 0)); self.aug = {}
+            self._clear_terms()
         return status
 
     def scan(self, u, z, R):

@@ -68,6 +68,37 @@ def test_reference_lands_on_oracle_map_scenario():
     assert ref.min_margin >= 1e-6
 
 
+def test_reference_lands_on_oracle_through_groups_and_a_reset():
+    """The input generator of tests/test_gpu_pipeline_componentwise.py on a small map: ghosts appended and matched in
+    the next scan, then a map reset and a rebuilt map that is re-observed.  The reference must agree with the
+    structured oracle's associations at every scan, stay within the bound, and keep every gate decision at least 1e-6
+    away from the threshold, so that the GPU cases rest on well-posed inputs."""
+    import ctypes
+    from oracle.oracle import StructuredOracle
+    import test_gpu_pipeline_componentwise as pc
+    c = pc.case_inputs("reset_small")
+    so, ref = StructuredOracle(c["cap"], reset_headroom=c["headroom"]), hp.HPFilter(c["cap"], reset_headroom=c["headroom"])
+    np.ctypeslib.as_array(so._lib.ekfo_y_ptr(so._h), shape=(so.n,))[:] = c["y"]
+    so.P_view()[:] = c["P"]
+    so._lib.ekfo_set_lines(so._h, ctypes.c_int(c["L"]))
+    so.set_pose(c["y"][:3])
+    ref.upload(c["y"], c["P"], c["L"])
+    lines, matched_new = [], 0
+    for s, (u, z, R) in enumerate(c["scans"]):
+        L_before = ref.L
+        st, jo = so.scan(u, z, R)
+        st2, jr = ref.scan(u, z, R)
+        assert np.array_equal(jo, jr) and st == st2, "scan %d: oracle %s, reference %s" % (s, jo, jr)
+        assert so.lines == ref.L, "scan %d" % s
+        if ref.L >= L_before and s:
+            matched_new += int((jr >= lines[-1][0]).sum()) if lines[-1][1] > lines[-1][0] else 0
+        lines.append((L_before, ref.L))
+    assert sum(a < b for b, a in lines) == 1, lines                                          # one reset
+    assert matched_new >= 8, "lines matched a landmark appended by the scan before: %d" % matched_new
+    _pin(so, ref, "groups and a reset")
+    assert ref.min_margin >= 1e-6
+
+
 def test_componentwise_check_flags_sweep_faults_the_normwise_check_misses():
     """One scan of 8 matched lines on a 94-landmark map (nl = 191: the last 64-column tile is one short of full),
     P spread over 10 decades, the last landmarks' entries the smallest.  Faults applied to the reference's own result:
