@@ -129,6 +129,17 @@ int ekf_get_ellipse(ekf_ctx* ctx, float axii[2], float* angle, int* ok);
 int ekf_download(ekf_ctx* ctx, double* y, double* P, int* n_lines);
 int ekf_upload(ekf_ctx* ctx, const double* y, const double* P, int n_lines);
 
+/* Map management, not in the reference.  Removes landmarks lines[0..k) (strictly increasing, each in
+ * [0, savedLineCount)) from the map: their entries of y and their rows and columns of P are deleted and the later
+ * landmarks move down in order (landmark j becomes j minus the number of removed indices below it) -- the marginal of
+ * the remaining state, pure data movement, bit for bit.  Waits for the sweep in flight.  *n_lines (nullable) = the new
+ * savedLineCount.  k = 0 is a no-op.  The caller chooses the indices (ekf_scan's j_out says which landmarks each scan
+ * matched); the library has no removal policy of its own, and the map reset of Robot.cpp:893-904 is unchanged.
+ * EKF_EINVAL: bad list (unsorted, duplicate, out of range, k < 0, NULL with k > 0), or a row-sharded filter (rows would
+ * move between ranks); EKF_ESTATE: inside an open step-wise scan.  On error the state is unchanged.  The Monte-Carlo
+ * batch filters (ekf_batch_*) have no such call. */
+int ekf_remove_lines(ekf_ctx* ctx, int k, const int* lines, int* n_lines);
+
 /* Live part only: nl = 3 + 2*savedLineCount entries of y and an nl x nl block with row stride ldp.
  * Fails with EKF_EINVAL if nl > max_n. */
 int ekf_download_live(ekf_ctx* ctx, double* y, double* P, int ldp, int max_n, int* n_lines);

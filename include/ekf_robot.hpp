@@ -121,6 +121,16 @@ class Robot {
     return msg;
   }
 
+  /* Not in the reference: removes landmarks `lines` (strictly increasing, each below savedLineCount) from the map
+   * (ekf_remove_lines) and updates savedLineCount.  A node can prune spurious or long-unseen landmarks with it instead of
+   * waiting for the reset of Robot.cpp:893-904.  lineIntervals is the per-scan log the node clears after publishing:
+   * untouched.  Returns the new savedLineCount; throws on a bad list. */
+  int removeLines(const std::vector<int>& lines) {
+    const int rc = ekf_remove_lines(ctx_, (int)lines.size(), lines.empty() ? 0 : lines.data(), &savedLineCount);
+    if (rc != EKF_OK) throw std::runtime_error(std::string("libekfcuda: ") + ekf_last_error(ctx_));
+    return savedLineCount;
+  }
+
   /* copies y and P_t0 back in the reference's layout (SLAMSIZE and SLAMSIZE^2 doubles) */
   void syncCovariance() {
     y.assign((size_t)n_, 0.0); P_t0.assign((size_t)n_ * n_, 0.0);

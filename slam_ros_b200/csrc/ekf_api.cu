@@ -123,6 +123,7 @@ struct ekf_ctx {
   /* staging for download / upload / stats */
   double* d_stage; size_t stage_elems;
   double* d_partials; double* d_out3;
+  int* d_keep;                /* ekf_remove_lines: old state index of every kept one (n ints, allocated on first use) */
   char err[256];
 };
 
@@ -636,7 +637,7 @@ int create_common(ekf_ctx** out, const ekf_config* cfg, int rank, int world, con
   ctx->stream = 0; ctx->max_lines = 0; ctx->d_in = 0; ctx->h_in = 0; ctx->h_jout = 0; ctx->h_st = 0;
   ctx->L_ub = 0; ctx->pend_ub = 0; ctx->scan_open = 0; ctx->cursor = 0;
   ctx->prof = 0; ctx->ev_used = 0; ctx->lev_used = 0; ctx->launches = 0; ctx->comm = 0; ctx->t0 = 0; ctx->t1 = 0;
-  ctx->d_stage = 0; ctx->stage_elems = 0; ctx->d_partials = 0; ctx->d_out3 = 0;
+  ctx->d_stage = 0; ctx->stage_elems = 0; ctx->d_partials = 0; ctx->d_out3 = 0; ctx->d_keep = 0;
   ctx->overlap = 0; ctx->wstream = 0; ctx->Pbuf[0] = ctx->Pbuf[1] = 0; ctx->rd = 0; ctx->par = 0; ctx->group = 8; ctx->tabpar = 0;
   { const char* e = getenv("EKF_CHUNK"); ctx->chunk_lines = e ? atoi(e) : 16; if (ctx->chunk_lines < 0) ctx->chunk_lines = 0; }
   { const char* e = getenv("EKF_FUSE_PREDICT"); ctx->no_fuse = (e && atoi(e) == 0) ? 1 : 0; }
@@ -873,7 +874,7 @@ int ekf_destroy(ekf_ctx* ctx) {
   if (ctx->evF[0]) cudaEventDestroy(ctx->evF[0]);
   if (ctx->evF[1]) cudaEventDestroy(ctx->evF[1]);
   if (ctx->wstream) cudaStreamDestroy(ctx->wstream);
-  cudaFree(ctx->d_stage); cudaFree(ctx->d_partials); cudaFree(ctx->d_out3);
+  cudaFree(ctx->d_stage); cudaFree(ctx->d_partials); cudaFree(ctx->d_out3); cudaFree(ctx->d_keep);
   cudaFreeHost(ctx->h_st); cudaFreeHost(ctx->h_snap);
   if (ctx->ev_snap) cudaEventDestroy(ctx->ev_snap);
   for (size_t i = 0; i < ctx->ev.size(); ++i) cudaEventDestroy(ctx->ev[i]);
@@ -1215,6 +1216,77 @@ int ekf_upload(ekf_ctx* ctx, const double* y, const double* P, int n_lines) {
   ctx->L_ub = n_lines;
   ctx->snap_inflight = 0;
   if (y && P) ctx->poisoned = 0;      /* a complete state replaces whatever a failed exchange left behind */
+  return EKF_OK;
+}
+
+/* Marginalising landmarks out of the Gaussian deletes their entries of y and their rows and columns of P: a gather of
+ * the kept entries, no arithmetic.  Hot storage goes through the stage; the cold upper triangle goes out of place into
+ * the second covariance buffer when there is one, else in place through the stage in batches of destination rows in
+ * increasing order: a later batch reads source rows keep[r] >= r, past every row already written, so the kernel
+ * boundaries are the only ordering needed. */
+int ekf_remove_lines(ekf_ctx* ctx, int k, const int* lines, int* n_lines) {
+  if (!ctx) return EKF_EINVAL;
+  if (k < 0 || (k > 0 && !lines)) { snprintf(ctx->err, sizeof ctx->err, "ekf_remove_lines: k = %d, lines = %p", k, (const void*)lines); return EKF_EINVAL; }
+  if (ctx->g.world > 1) {
+    snprintf(ctx->err, sizeof ctx->err, "ekf_remove_lines: not supported on a row-sharded filter (rows would move between ranks)");
+    return EKF_EINVAL;
+  }
+  if (ctx->scan_open) { snprintf(ctx->err, sizeof ctx->err, "ekf_remove_lines inside an open scan"); return EKF_ESTATE; }
+  NOT_POISONED(ctx);
+  CU(cudaSetDevice(ctx->cfg.device));
+  int rc = read_state(ctx);               /* the exact line count; nothing is changed before the list is validated */
+  if (rc) return rc;
+  const int L = ctx->h_st->L;
+  for (int i = 0; i < k; ++i)
+    if (lines[i] < 0 || lines[i] >= L || (i > 0 && lines[i] <= lines[i - 1])) {
+      snprintf(ctx->err, sizeof ctx->err, "ekf_remove_lines: lines[%d] = %d (need strictly increasing indices in [0, %d))", i, lines[i], L);
+      return EKF_EINVAL;
+    }
+  if (k == 0) { if (n_lines) *n_lines = L; return EKF_OK; }
+  rc = drain(ctx);                        /* no sweep in flight, no open group: Pbuf[rd] is the one complete covariance */
+  if (rc) return rc;
+  const int Ln = L - k, nl = 3 + 2 * Ln;
+  std::vector<int> keep((size_t)nl);
+  for (int i = 0; i < 3; ++i) keep[i] = i;
+  for (int j = 0, t = 0, jn = 0; j < L; ++j) {
+    if (t < k && lines[t] == j) { ++t; continue; }
+    keep[3 + 2 * jn] = 3 + 2 * j; keep[4 + 2 * jn] = 4 + 2 * j; ++jn;
+  }
+  if (!ctx->d_keep) CU(cudaMalloc(&ctx->d_keep, (size_t)ctx->g.n * sizeof(int)));
+  CU(cudaMemcpyAsync(ctx->d_keep, keep.data(), (size_t)nl * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+  const size_t hot = 6 * (size_t)nl - 6;
+  size_t rows_per = kStageElems / (size_t)nl;
+  if (rows_per < 1) rows_per = 1;
+  if (rows_per > (size_t)nl) rows_per = nl;
+  rc = ensure_stage(ctx, hot > rows_per * nl ? hot : rows_per * nl);
+  if (rc) return rc;
+  CU(ekf_launch_remove_hot(ctx->g, ctx->b, ctx->d_keep, nl, ctx->d_stage, 0, ctx->stream));
+  CU(ekf_launch_remove_hot(ctx->g, ctx->b, ctx->d_keep, nl, ctx->d_stage, 1, ctx->stream));
+  const size_t ld = ctx->g.ld;
+  if (ctx->overlap) {                     /* out of place: Pbuf[rd] -> Pbuf[rd ^ 1], which becomes the line stream's buffer */
+    const int dst = ctx->rd ^ 1;
+    CU(ekf_launch_remove_cold(ctx->Pbuf[ctx->rd], ld, 0, ctx->Pbuf[dst], ld, 0, ctx->d_keep, 3, nl - 3, nl, 0, ctx->stream));
+    ctx->rd = dst;
+    ctx->b.P = ctx->Pbuf[ctx->rd];
+    ctx->launches += 3;
+  } else {
+    /* in place: rows and columns before the first removed index keep their place, so rows above it only move their
+     * columns from it on */
+    const int f = 3 + 2 * lines[0];
+    for (int r0 = 3; r0 < nl; r0 += (int)rows_per) {
+      const int cnt = nl - r0 < (int)rows_per ? nl - r0 : (int)rows_per;
+      CU(ekf_launch_remove_cold(ctx->b.P, ld, 0, ctx->d_stage, (size_t)nl, r0, ctx->d_keep, r0, cnt, nl, f, ctx->stream));
+      CU(ekf_launch_remove_cold(ctx->d_stage, (size_t)nl, r0, ctx->b.P, ld, 0, 0, r0, cnt, nl, f, ctx->stream));
+      ctx->launches += 2;
+    }
+    ctx->launches += 2;
+  }
+  ctx->h_st->L = Ln;
+  CU(cudaMemcpyAsync(&ctx->b.st->L, &ctx->h_st->L, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  ctx->L_ub = Ln;
+  ctx->snap_inflight = 0;
+  if (n_lines) *n_lines = Ln;
   return EKF_OK;
 }
 

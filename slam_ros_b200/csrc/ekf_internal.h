@@ -133,6 +133,15 @@ cudaError_t ekf_launch_scatter(const EkfGeom& g, const EkfBuffers& b, int r0, in
 cudaError_t ekf_launch_cov_stats(const EkfGeom& g, const EkfBuffers& b, double* d_partials, int n_partials,
                                  double* d_out3, cudaStream_t s);
 cudaError_t ekf_launch_zero_pending(const EkfGeom& g, const EkfBuffers& b, int m, int* d_np, cudaStream_t s);
+/* landmark removal (ekf_remove_lines), keep[i] = old state index of new state index i < nl (strictly increasing).
+ * hot: y, rows 0..2 of top and the 2x2 diagonal blocks into stage ((6 nl - 6) doubles, put = 0), then back (put = 1);
+ * cold: destination rows [r0, r0 + nr) of the live upper triangle from column max(r, c_from) on; row r lives at
+ * dst + (r - dst_row0) * ld_dst and reads source row keep[r] (keep = NULL: row r) at src + (row - src_row0) * ld_src,
+ * columns keep[c] (keep = NULL: c).  Single-GPU layout only. */
+cudaError_t ekf_launch_remove_hot(const EkfGeom& g, const EkfBuffers& b, const int* keep, int nl, double* stage, int put,
+                                  cudaStream_t s);
+cudaError_t ekf_launch_remove_cold(const double* src, size_t ld_src, int src_row0, double* dst, size_t ld_dst, int dst_row0,
+                                   const int* keep, int r0, int nr, int nl, int c_from, cudaStream_t s);
 int ekf_sweep_grid_ub(const EkfGeom& g, int L_ub);
 
 /* The largest double T with sqrt(T) <= gate (sqrt correctly rounded): Robot.cpp:489's `sqrt(fabs(d2)) > MAHALANOBIS`

@@ -1755,6 +1755,61 @@ __global__ void k_zero_pending(EkfGeom g, EkfBuffers b, int m, int* np) {
   if (blockIdx.x == 0 && threadIdx.x == 0) *np = m;
 }
 
+/* ------------------------------------------------------------------------------------------------ */
+/* Landmark removal (ekf_remove_lines, DESIGN section 3): pure data movement.  keep[i] = old state index of new state
+ * index i (i < nl, strictly increasing, keep[i] = i for i < 3). */
+
+/* Hot storage: y, rows 0..2 of `top` and the 2x2 diagonal blocks of the kept landmarks.  put = 0 gathers them into
+ * stage = [y (nl) | top rows (3 x nl) | diag (4 x L)]; put = 1 copies the stage back in place (the two launches are the
+ * ordering: a kept entry's source may be another kept entry's destination). */
+__global__ void __launch_bounds__(EKF_BLOCK) k_remove_hot(EkfGeom g, EkfBuffers b, const int* __restrict__ keep, int nl,
+                                                          double* __restrict__ stage, int put) {
+  const long long total = 4LL * nl + 2LL * (nl - 3);
+  for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < total; t += (long long)gridDim.x * blockDim.x) {
+    double* dst;
+    const double* src;
+    if (t < nl) { dst = b.y + t; src = b.y + keep[t]; }
+    else if (t < 4LL * nl) {
+      const int k = (int)((t - nl) / nl), c = (int)((t - nl) % nl);
+      dst = b.top + (size_t)k * g.ld + c; src = b.top + (size_t)k * g.ld + keep[c];
+    } else {
+      const int e = (int)(t - 4LL * nl), j = e >> 2, w = e & 3;
+      dst = b.diag + 4 * j + w; src = b.diag + 4 * ((keep[3 + 2 * j] - 3) >> 1) + w;
+    }
+    if (put) *dst = stage[t]; else stage[t] = *src;
+  }
+}
+
+/* Cold covariance, rows [r0, r0 + nr) of the compacted live upper triangle.  Destination row r (at dst + (r - dst_row0) *
+ * ld_dst) gets, in columns max(r, c_from) .. nl-1, the source elements (keep[r], keep[c]) (GATHER) or (r, c) (the copy back
+ * from the stage), source row i at src + (i - src_row0) * ld_src.  keep is increasing, so an upper destination element
+ * has an upper source.  The kept runs between removed landmarks make each row's reads piecewise contiguous: one CTA per
+ * row, RM_UNROLL independent 8-byte loads in flight per thread, read-once data streamed past L1/L2 (ld.cs / st.cs). */
+#define RM_UNROLL 4
+template <bool GATHER>
+__global__ void __launch_bounds__(EKF_BLOCK) k_remove_cold(const double* __restrict__ src, size_t ld_src, int src_row0,
+                                                           double* __restrict__ dst, size_t ld_dst, int dst_row0,
+                                                           const int* __restrict__ keep, int r0, int nr, int nl, int c_from) {
+  for (int i = blockIdx.x; i < nr; i += gridDim.x) {
+    const int r = r0 + i;
+    const double* s = src + (size_t)((GATHER ? __ldg(keep + r) : r) - src_row0) * ld_src;
+    double* d = dst + (size_t)(r - dst_row0) * ld_dst;
+    for (int c = max(r, c_from) + threadIdx.x; c < nl; c += RM_UNROLL * EKF_BLOCK) {
+      double v[RM_UNROLL];
+#pragma unroll
+      for (int u = 0; u < RM_UNROLL; ++u) {
+        const int cc = c + u * EKF_BLOCK;
+        if (cc < nl) v[u] = __ldcs(s + (GATHER ? __ldg(keep + cc) : cc));
+      }
+#pragma unroll
+      for (int u = 0; u < RM_UNROLL; ++u) {
+        const int cc = c + u * EKF_BLOCK;
+        if (cc < nl) __stcs(d + cc, v[u]);
+      }
+    }
+  }
+}
+
 inline int blocks_for(long long n, int cap = 1 << 20) {
   long long bl = (n + EKF_BLOCK - 1) / EKF_BLOCK;
   if (bl < 1) bl = 1;
@@ -2120,6 +2175,18 @@ cudaError_t ekf_launch_cov_stats(const EkfGeom& g, const EkfBuffers& b, double* 
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return e;
   k_cov_fold<<<1, 32, 0, s>>>(b, d_partials, d_out3);
+  return cudaGetLastError();
+}
+cudaError_t ekf_launch_remove_hot(const EkfGeom& g, const EkfBuffers& b, const int* keep, int nl, double* stage, int put,
+                                  cudaStream_t s) {
+  k_remove_hot<<<blocks_for(6LL * nl, 148 * 8), EKF_BLOCK, 0, s>>>(g, b, keep, nl, stage, put);
+  return cudaGetLastError();
+}
+cudaError_t ekf_launch_remove_cold(const double* src, size_t ld_src, int src_row0, double* dst, size_t ld_dst, int dst_row0,
+                                   const int* keep, int r0, int nr, int nl, int c_from, cudaStream_t s) {
+  if (nr <= 0) return cudaSuccess;
+  if (keep) k_remove_cold<true><<<nr, EKF_BLOCK, 0, s>>>(src, ld_src, src_row0, dst, ld_dst, dst_row0, keep, r0, nr, nl, c_from);
+  else k_remove_cold<false><<<nr, EKF_BLOCK, 0, s>>>(src, ld_src, src_row0, dst, ld_dst, dst_row0, keep, r0, nr, nl, c_from);
   return cudaGetLastError();
 }
 cudaError_t ekf_launch_zero_pending(const EkfGeom& g, const EkfBuffers& b, int m, int* d_np, cudaStream_t s) {

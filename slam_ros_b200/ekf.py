@@ -44,7 +44,7 @@ def library_path():
 SYMBOLS = [
     "ekf_default_config", "ekf_create", "ekf_destroy", "ekf_last_error", "ekf_predict", "ekf_associate",
     "ekf_update", "ekf_add_line", "ekf_end_scan", "ekf_scan", "ekf_scan_device", "ekf_sync", "ekf_get_state",
-    "ekf_get_robot_cov", "ekf_get_ellipse", "ekf_download", "ekf_upload", "ekf_download_live",
+    "ekf_get_robot_cov", "ekf_get_ellipse", "ekf_download", "ekf_upload", "ekf_remove_lines", "ekf_download_live",
     "ekf_download_block", "ekf_cov_stats", "ekf_profile_enable", "ekf_profile_read", "ekf_profile_read_lines", "ekf_timer_start", "ekf_timer_stop", "ekf_sweep_probe",
     "ekf_nccl_unique_id", "ekf_create_sharded", "ekf_shard_ipc_handle", "ekf_shard_connect", "ekf_shard_use_fused", "ekf_batch_create", "ekf_batch_destroy", "ekf_batch_scan",
     "ekf_batch_submit", "ekf_batch_collect", "ekf_batch_scan_device", "ekf_batch_sync", "ekf_batch_download", "ekf_batch_last_error", "ekf_version",
@@ -88,6 +88,7 @@ def load_library():
     lib.ekf_get_ellipse.argtypes = [vp, _fp, _fp, _ip]
     lib.ekf_download.argtypes = [vp, _dp, _dp, _ip]
     lib.ekf_upload.argtypes = [vp, _dp, _dp, C.c_int]
+    lib.ekf_remove_lines.argtypes = [vp, C.c_int, _ip, _ip]
     lib.ekf_download_live.argtypes = [vp, _dp, _dp, C.c_int, C.c_int, _ip]
     lib.ekf_download_block.argtypes = [vp, C.c_int, C.c_int, C.c_int, C.c_int, _dp]
     lib.ekf_cov_stats.argtypes = [vp, _dp, _dp, _dp]
@@ -304,6 +305,15 @@ class EkfFilter:
     def upload(self, y, P, n_lines):
         ya = _arr(y, (self.n,)); Pa = _arr(P, (self.n, self.n))
         self._check(self._lib.ekf_upload(self._h, _p(ya), _p(Pa), int(n_lines)), "ekf_upload")
+
+    def remove_lines(self, indices):
+        """Removes landmarks `indices` (strictly increasing, each below the line count) from the map: their entries of y
+        and rows and columns of P go, later landmarks move down in order.  Returns the new line count."""
+        idx = np.ascontiguousarray(np.asarray(indices, dtype=np.int32).reshape(-1))
+        L = C.c_int(0)
+        self._check(self._lib.ekf_remove_lines(self._h, idx.size, idx.ctypes.data_as(_ip) if idx.size else None,
+                                               C.byref(L)), "ekf_remove_lines")
+        return int(L.value)
 
     def cov_stats(self):
         t = C.c_double(0); s = C.c_double(0); q = C.c_double(0)

@@ -116,6 +116,12 @@ class Robot:
                     self.lineIntervals.extend(interval_end_point(alpha, rr, self.xPos, self.yPos, self.thetaPos))
         return rc
 
+    def remove_lines(self, indices):
+        """Not in the reference: removes landmarks `indices` (strictly increasing) from the map (ekf_remove_lines).
+        savedLineCount follows; lineIntervals, the per-scan log the node clears after publishing, is untouched.
+        Returns the new savedLineCount."""
+        return self._f.remove_lines(indices)
+
     def getEllipse(self):
         """Robot::getEllipse (Robot.cpp:73-124) -> (ok, (axis0, axis1), angle)."""
         return self._f.get_ellipse()
