@@ -140,6 +140,25 @@ int ekf_upload(ekf_ctx* ctx, const double* y, const double* P, int n_lines);
  * batch filters (ekf_batch_*) have no such call. */
 int ekf_remove_lines(ekf_ctx* ctx, int k, const int* lines, int* n_lines);
 
+/* Absolute pose measurement, not in the reference (GNSS, UWB, motion capture, a docking fiducial, a relocaliser).
+ * mask selects d = popcount(mask) components of the pose; z is a full 3-vector (x, y, theta) and R a full row-major 3x3
+ * covariance, of which only the selected entries are read.  With H = the selected rows of [I_3 0]:
+ *   v = z_sel - y_sel (the theta component wrapped by normalize_radian, Robot.cpp:62-71), S = H P H' + R_sel (from the
+ *   upper triangle), S^-1 by LU with partial pivoting, d2 = v' S^-1 v, K = P H' S^-1, P -= (K S) K', y += K v, then
+ *   normalize_radian(y[2]); the pose (xPos, yPos, thetaPos) and x_pre follow y[0:3], as after a line update
+ *   (Robot.cpp:516-602 with d x d blocks).
+ * The fix is accepted iff S is nonsingular and d2 <= d2_max (a chi-square threshold for d degrees of freedom; +inf
+ * accepts everything, a NaN d2 is rejected).  A rejected fix leaves the state bit for bit unchanged and returns EKF_OK
+ * with *accepted = 0; a singular S (e.g. theta alone on a fresh filter, P[2,2] = 0, with R_thth = 0) returns
+ * EKF_ESINGULAR, state unchanged.  d2, accepted and pose (the resulting xPos, yPos, thetaPos) are nullable; when all three
+ * are NULL the call returns after enqueueing and a singular S is not reported.  Waits for the sweep in flight.
+ * EKF_EINVAL: mask 0 or above 7, NULL z or R, a non-finite selected entry, a selected R that is not symmetric, a NaN
+ * d2_max, or a row-sharded filter; EKF_ESTATE: inside an open step-wise scan.  On error the state is unchanged.  The
+ * Monte-Carlo batch filters (ekf_batch_*) have no such call. */
+enum { EKF_POSE_X = 1, EKF_POSE_Y = 2, EKF_POSE_THETA = 4 };
+int ekf_observe_pose(ekf_ctx* ctx, int mask, const double z[3], const double R[9], double d2_max, double* d2,
+                     int* accepted, double pose[3]);
+
 /* Live part only: nl = 3 + 2*savedLineCount entries of y and an nl x nl block with row stride ldp.
  * Fails with EKF_EINVAL if nl > max_n. */
 int ekf_download_live(ekf_ctx* ctx, double* y, double* P, int ldp, int max_n, int* n_lines);

@@ -131,6 +131,22 @@ class Robot {
     return savedLineCount;
   }
 
+  /* Not in the reference: fuses an absolute pose measurement (ekf_observe_pose): z = (x, y, theta), R its row-major 3x3
+   * covariance, mask of EKF_POSE_X | EKF_POSE_Y | EKF_POSE_THETA (only the selected entries are read), accepted iff S
+   * is nonsingular and d2 <= d2Max.  xPos / yPos / thetaPos follow the corrected pose: localize passes them as x_t0
+   * (Robot.cpp:130), so a stale mirror would undo the fix at the next prediction.  As after any update, the next localize
+   * forms its odometry from the corrected pose and the encoder pose (Robot.cpp:140-145).  Returns whether the fix was
+   * accepted (d2 nullable); a singular S returns false with the state unchanged; throws on bad arguments. */
+  bool observePose(const double z[3], const double R[9], int mask = EKF_POSE_X | EKF_POSE_Y | EKF_POSE_THETA,
+                   double d2Max = HUGE_VAL, double* d2 = 0) {
+    int accepted = 0;
+    double pose[3];
+    const int rc = ekf_observe_pose(ctx_, mask, z, R, d2Max, d2, &accepted, pose);
+    if (rc != EKF_OK && rc != EKF_ESINGULAR) throw std::runtime_error(std::string("libekfcuda: ") + ekf_last_error(ctx_));
+    xPos = pose[0]; yPos = pose[1]; thetaPos = pose[2];
+    return accepted != 0;
+  }
+
   /* copies y and P_t0 back in the reference's layout (SLAMSIZE and SLAMSIZE^2 doubles) */
   void syncCovariance() {
     y.assign((size_t)n_, 0.0); P_t0.assign((size_t)n_ * n_, 0.0);

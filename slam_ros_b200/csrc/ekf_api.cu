@@ -1290,6 +1290,75 @@ int ekf_remove_lines(ekf_ctx* ctx, int k, const int* lines, int* n_lines) {
   return EKF_OK;
 }
 
+/* An absolute pose fix is a rank-d (d <= 3) update whose gain needs only P[:, 0:3], which is hot storage and current at
+ * all times.  The call drains first (no open sweep group, no sweep in flight: Pbuf[rd] is the one complete covariance),
+ * then enqueues the gain, the hot update and one in-place sweep of (at most) two rank-2 terms.  A rejected fix or a
+ * singular S leaves st->np = 0, and every sweep form returns without writing for a zero count: the state is unchanged. */
+int ekf_observe_pose(ekf_ctx* ctx, int mask, const double z[3], const double R[9], double d2_max, double* d2,
+                     int* accepted, double pose[3]) {
+  if (!ctx) return EKF_EINVAL;
+  if (mask < 1 || mask > 7 || !z || !R || d2_max != d2_max) {
+    snprintf(ctx->err, sizeof ctx->err, "ekf_observe_pose: mask = %d, z = %p, R = %p, d2_max = %g", mask, (const void*)z,
+             (const void*)R, d2_max);
+    return EKF_EINVAL;
+  }
+  EkfPoseFix f;
+  memset(&f, 0, sizeof f);
+  int d = 0;
+  for (int c = 0; c < 3; ++c) if (mask & (1 << c)) f.sel[d++] = c;
+  for (int i = 0; i < d; ++i) {
+    f.z[i] = z[f.sel[i]];
+    if (!isfinite(f.z[i])) { snprintf(ctx->err, sizeof ctx->err, "ekf_observe_pose: z[%d] is not finite", f.sel[i]); return EKF_EINVAL; }
+    for (int k = 0; k < d; ++k) {
+      const int r = f.sel[i], c = f.sel[k];
+      f.R[3 * i + k] = R[3 * r + c];
+      if (!isfinite(R[3 * r + c]) || R[3 * r + c] != R[3 * c + r]) {
+        snprintf(ctx->err, sizeof ctx->err, "ekf_observe_pose: R[%d][%d] = %g is not finite or not symmetric", r, c, R[3 * r + c]);
+        return EKF_EINVAL;
+      }
+    }
+  }
+  f.d2max = d2_max;
+  if (ctx->g.world > 1) {
+    snprintf(ctx->err, sizeof ctx->err, "ekf_observe_pose: not supported on a row-sharded filter");
+    return EKF_EINVAL;
+  }
+  if (ctx->scan_open) { snprintf(ctx->err, sizeof ctx->err, "ekf_observe_pose inside an open scan"); return EKF_ESTATE; }
+  NOT_POISONED(ctx);
+  CU(cudaSetDevice(ctx->cfg.device));
+  int rc = drain(ctx);
+  if (rc) return rc;
+  /* term 2 goes to slot 1; with a single slot (max_batch = 1) to a scratch row, folded by a second one-term sweep */
+  const bool one_slot = ctx->slots < 2;
+  const size_t ld = ctx->g.ld;
+  if (one_slot) { rc = ensure_stage(ctx, 4 * ld); if (rc) return rc; }
+  double2* K2 = one_slot ? (double2*)ctx->d_stage : ctx->b.Kp + ld;
+  double2* KS2 = one_slot ? (double2*)ctx->d_stage + ld : ctx->b.KSp + ld;
+  CU(ekf_launch_pose_gain(ctx->g, ctx->b, f, d, K2, KS2, ctx->L_ub, ctx->stream));
+  CU(ekf_launch_pose_apply(ctx->g, ctx->b, d, K2, KS2, one_slot ? 1 : 2, ctx->L_ub, ctx->stream));
+  ctx->launches += 2;
+  rc = sweep_now(ctx, (d == 3 && !one_slot) ? 2 : 1);
+  if (rc) return rc;
+  if (one_slot && d == 3) {
+    CU(ekf_launch_pose_term2(ctx->g, ctx->b, d, K2, KS2, ctx->L_ub, ctx->stream));
+    ctx->launches++;
+    rc = sweep_now(ctx, 1);
+    if (rc) return rc;
+  }
+  if (!d2 && !accepted && !pose) return EKF_OK;
+  rc = read_state(ctx);
+  if (rc) return rc;
+  const int st = ctx->h_st->fix_status;
+  if (d2) *d2 = ctx->h_st->fix_d2;
+  if (accepted) *accepted = st == EKF_FIX_ACCEPTED;
+  if (pose) memcpy(pose, ctx->h_st->pose, 3 * sizeof(double));
+  if (st == EKF_FIX_SINGULAR) {
+    snprintf(ctx->err, sizeof ctx->err, "ekf_observe_pose: S is singular (mask %d); the state is unchanged", mask);
+    return EKF_ESINGULAR;
+  }
+  return EKF_OK;
+}
+
 int ekf_cov_stats(ekf_ctx* ctx, double* trace, double* sum, double* sumsq) {
   if (!ctx) return EKF_EINVAL;
   if (ctx->scan_open) return EKF_ESTATE;

@@ -98,6 +98,74 @@ __device__ __forceinline__ int inv2x2_lu(const double S[4], double Si[4]) {
   return 0;
 }
 
+/* The D x D generalisation of inv2x2_lu (D <= 3, row stride 3): gsl_linalg_LU_decomp (first-largest partial pivot,
+ * elimination skipped on a zero pivot) then gsl_linalg_LU_invert, one column of the identity at a time: permute, unit
+ * lower forward substitution, upper back substitution, in the reference-BLAS dtrsv order.  Returns 1 (Si = 0) when a
+ * diagonal entry of U is zero, as LU_invert's singularity test does. */
+template <int D>
+__device__ __forceinline__ int invDxD_lu(const double S[9], double Si[9]) {
+  double a[D][D];
+  int p[D];
+#pragma unroll
+  for (int i = 0; i < D; ++i) {
+    p[i] = i;
+#pragma unroll
+    for (int k = 0; k < D; ++k) a[i][k] = S[3 * i + k];
+  }
+#pragma unroll
+  for (int j = 0; j < D - 1; ++j) {
+    double mx = fabs(a[j][j]);
+    int piv = j;
+#pragma unroll
+    for (int i = j + 1; i < D; ++i) if (fabs(a[i][j]) > mx) { mx = fabs(a[i][j]); piv = i; }
+#pragma unroll
+    for (int i = j + 1; i < D; ++i)             /* swap rows j and piv (register arrays: select, no dynamic index) */
+      if (piv == i) {
+#pragma unroll
+        for (int k = 0; k < D; ++k) { const double t = a[j][k]; a[j][k] = a[i][k]; a[i][k] = t; }
+        const int t = p[j]; p[j] = p[i]; p[i] = t;
+      }
+    const double ajj = a[j][j];
+    if (ajj != 0.0) {
+#pragma unroll
+      for (int i = j + 1; i < D; ++i) {
+        const double l = __ddiv_rn(a[i][j], ajj);
+        a[i][j] = l;
+#pragma unroll
+        for (int k = j + 1; k < D; ++k) a[i][k] = sub_rn(a[i][k], mul_rn(l, a[j][k]));
+      }
+    }
+  }
+  bool sing = false;
+#pragma unroll
+  for (int i = 0; i < D; ++i) sing = sing || a[i][i] == 0.0;
+  if (sing) {
+#pragma unroll
+    for (int t = 0; t < 9; ++t) Si[t] = 0.0;
+    return 1;
+  }
+#pragma unroll
+  for (int col = 0; col < D; ++col) {
+    double x[D];
+#pragma unroll
+    for (int i = 0; i < D; ++i) x[i] = (p[i] == col) ? 1.0 : 0.0;
+#pragma unroll
+    for (int i = 1; i < D; ++i)                                        /* L x = P e (unit diagonal) */
+#pragma unroll
+      for (int k = 0; k < i; ++k) x[i] = sub_rn(x[i], mul_rn(a[i][k], x[k]));
+    x[D - 1] = __ddiv_rn(x[D - 1], a[D - 1][D - 1]);                   /* U x = . */
+#pragma unroll
+    for (int i = D - 2; i >= 0; --i) {
+      double t = x[i];
+#pragma unroll
+      for (int k = i + 1; k < D; ++k) t = sub_rn(t, mul_rn(a[i][k], x[k]));
+      x[i] = __ddiv_rn(t, a[i][i]);
+    }
+#pragma unroll
+    for (int i = 0; i < D; ++i) Si[3 * i + col] = x[i];
+  }
+  return 0;
+}
 
 /* Robot.cpp:367-489 for one (line, landmark) pair, given P gathered at rows/cols {0,1,2,a,b} (Cm), the
  * landmark (m0, m1) = (y[a], y[b]), the predicted pose, the observed line z and its covariance R.

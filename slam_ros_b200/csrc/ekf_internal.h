@@ -44,7 +44,20 @@ struct EkfDevState {          /* one per filter, in global memory */
   int np;                     /* pending rank-2 terms = pidx[line] - pbase */
   int xseq;                   /* row-sharded mode: matched lines exchanged over NVLink so far (same on every rank) */
   int L0;                     /* savedLineCount before the last end-of-scan's append (read by its phase B) */
+  /* the last absolute pose fix (ekf_observe_pose, d = its component count): decision and diagnostic tap */
+  int fix_status;             /* EKF_FIX_* */
+  double fix_S[9];            /* S = H P H' + R_sel, d x d with row stride 3 */
+  double fix_v[3];            /* innovation z_sel - y_sel, theta wrapped */
+  double fix_d2;              /* v' S^-1 v */
 };
+#define EKF_FIX_REJECTED 0
+#define EKF_FIX_ACCEPTED 1
+#define EKF_FIX_SINGULAR 2
+
+/* one absolute pose fix, by value in the kernel parameters (compacted on the host, so that the kernels index it with
+ * constants only): sel[0..d) = the selected state indices (0 x, 1 y, 2 theta) in increasing order, z = z_sel, R = R_sel
+ * (d x d, row stride 3) */
+struct EkfPoseFix { double z[3]; double R[9]; double d2max; int sel[3]; };
 
 /* what a scan's (possibly later, possibly concurrent) sweep needs to know about that scan */
 struct EkfScanView { int cnt; int L; int pad[2]; };
@@ -142,6 +155,17 @@ cudaError_t ekf_launch_remove_hot(const EkfGeom& g, const EkfBuffers& b, const i
                                   cudaStream_t s);
 cudaError_t ekf_launch_remove_cold(const double* src, size_t ld_src, int src_row0, double* dst, size_t ld_dst, int dst_row0,
                                    const int* keep, int r0, int nr, int nl, int c_from, cudaStream_t s);
+/* absolute pose fix (ekf_observe_pose), d = 1..3 selected components, on the complete in-place covariance.
+ * gain: S, S^-1, v, d2 and the decision (into st->fix_*), and the gain rows as two rank-2 terms: term 1
+ * (K_0, K_1 ; KS_0, KS_1) into pending slot 0, term 2 (K_2, 0 ; KS_2, 0) into (K2, KS2) (slot 1, or a scratch row when
+ * there is one slot).  apply: the hot update, y, pose and x_pre, and st->np = the terms the sweep folds (0 when rejected;
+ * at most max_np).  term2: copies (K2, KS2) into slot 0 and sets st->np for a second one-term sweep (one slot only). */
+cudaError_t ekf_launch_pose_gain(const EkfGeom& g, const EkfBuffers& b, const EkfPoseFix& f, int d, double2* K2,
+                                 double2* KS2, int L_ub, cudaStream_t s);
+cudaError_t ekf_launch_pose_apply(const EkfGeom& g, const EkfBuffers& b, int d, const double2* K2, const double2* KS2,
+                                  int max_np, int L_ub, cudaStream_t s);
+cudaError_t ekf_launch_pose_term2(const EkfGeom& g, const EkfBuffers& b, int d, const double2* K2, const double2* KS2,
+                                  int L_ub, cudaStream_t s);
 int ekf_sweep_grid_ub(const EkfGeom& g, int L_ub);
 
 /* The largest double T with sqrt(T) <= gate (sqrt correctly rounded): Robot.cpp:489's `sqrt(fabs(d2)) > MAHALANOBIS`

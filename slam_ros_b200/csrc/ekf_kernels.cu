@@ -1810,6 +1810,164 @@ __global__ void __launch_bounds__(EKF_BLOCK) k_remove_cold(const double* __restr
   }
 }
 
+/* ------------------------------------------------------------------------------------------------ */
+/* Absolute pose fix (ekf_observe_pose, DESIGN section 3.2).  H = the D selected rows of [I_3 0], so P H' is D columns of
+ * P among 0..2 -- all in `top`, hot and always current -- and H P H' is a D x D block of the robot rows.  The arithmetic is
+ * the reference-BLAS pattern of Robot.cpp:516-602 with D x D blocks: PHt = P H', S = H P H' + R, S^-1 by LU, d2 = v' S^-1 v
+ * (TN then NN as at :479-483), K = PHt S^-1 and KS = K S (NN), P -= KS K' as two rank-2 terms, y += K v, then the wrap
+ * of y[2] and the pose mirrors (:596-602).  Products with the structural 0 / 1 entries of H are exact and not issued. */
+struct PoseGate { double S[9], Si[9], v[3], d2; int status; };
+
+template <int D>
+__device__ __forceinline__ void pose_gate(const EkfGeom& g, const EkfBuffers& b, const EkfPoseFix& f, PoseGate& G) {
+#pragma unroll
+  for (int i = 0; i < D; ++i)
+#pragma unroll
+    for (int k = 0; k < D; ++k) {                                     /* upper triangle of the robot block, plus R_sel */
+      const int r = min(f.sel[i], f.sel[k]), c = max(f.sel[i], f.sel[k]);
+      G.S[3 * i + k] = add_rn(b.top[(size_t)r * g.ld + c], f.R[3 * i + k]);
+    }
+  const int sing = invDxD_lu<D>(G.S, G.Si);
+#pragma unroll
+  for (int i = 0; i < D; ++i) {
+    double v = sub_rn(f.z[i], b.y[f.sel[i]]);
+    if (f.sel[i] == 2) normalize_radian(v);
+    G.v[i] = v;
+  }
+  double w[D];                                                        /* v' S^-1 (TN) */
+#pragma unroll
+  for (int c = 0; c < D; ++c) w[c] = 0.0;
+#pragma unroll
+  for (int k = 0; k < D; ++k)
+#pragma unroll
+    for (int c = 0; c < D; ++c) axpy_skip(w[c], G.v[k], G.Si[3 * k + c]);
+  double d2 = 0.0;                                                    /* (v' S^-1) v (NN) */
+#pragma unroll
+  for (int c = 0; c < D; ++c) axpy_skip(d2, w[c], G.v[c]);
+  G.d2 = d2;
+  /* accepted iff S is nonsingular and d2 <= d2max (false for a NaN d2) */
+  G.status = sing ? EKF_FIX_SINGULAR : (d2 <= f.d2max ? EKF_FIX_ACCEPTED : EKF_FIX_REJECTED);
+}
+
+/* Every block forms the gate redundantly (a few hundred flops); block 0 publishes it.  Each thread then writes the gain
+ * rows of its state indices as term 1 (slot 0) and, for D = 3, term 2 (K2, KS2). */
+template <int D>
+__global__ void __launch_bounds__(EKF_BLOCK) k_pose_gain(EkfGeom g, EkfBuffers b, EkfPoseFix f, double2* __restrict__ K2,
+                                                         double2* __restrict__ KS2) {
+  __shared__ PoseGate sG;
+  EkfDevState* st = b.st;
+  if (threadIdx.x == 0) {
+    pose_gate<D>(g, b, f, sG);
+    if (blockIdx.x == 0) {
+      st->fix_status = sG.status;
+      for (int t = 0; t < 9; ++t) st->fix_S[t] = (t / 3 < D && t % 3 < D) ? sG.S[t] : 0.0;
+      for (int t = 0; t < 3; ++t) st->fix_v[t] = t < D ? sG.v[t] : 0.0;
+      st->fix_d2 = sG.d2;
+    }
+  }
+  __syncthreads();
+  if (sG.status != EKF_FIX_ACCEPTED) return;
+  const int nl = 3 + 2 * st->L;
+  for (int r = blockIdx.x * blockDim.x + threadIdx.x; r < nl; r += gridDim.x * blockDim.x) {
+    double ph[D];                                                     /* P H': P[r, sel[i]] through the upper storage */
+#pragma unroll
+    for (int i = 0; i < D; ++i) ph[i] = b.top[(size_t)min(r, f.sel[i]) * g.ld + max(r, f.sel[i])];
+    double k[D], ks[D];
+#pragma unroll
+    for (int c = 0; c < D; ++c) { k[c] = 0.0; ks[c] = 0.0; }
+#pragma unroll
+    for (int i = 0; i < D; ++i)                                       /* K = PHt S^-1 (NN) */
+#pragma unroll
+      for (int c = 0; c < D; ++c) axpy_skip(k[c], ph[i], sG.Si[3 * i + c]);
+#pragma unroll
+    for (int i = 0; i < D; ++i)                                       /* K S (NN) */
+#pragma unroll
+      for (int c = 0; c < D; ++c) axpy_skip(ks[c], k[i], sG.S[3 * i + c]);
+    b.Kp[r] = make_double2(k[0], D > 1 ? k[1] : 0.0);
+    b.KSp[r] = make_double2(ks[0], D > 1 ? ks[1] : 0.0);
+    if (D == 3) { K2[r] = make_double2(k[D - 1], 0.0); KS2[r] = make_double2(ks[D - 1], 0.0); }
+  }
+}
+
+/* P -= KS K' on the hot elements (rows 0..2, the 2x2 diagonal blocks), term 1 then term 2 as the sweep folds them into the
+ * cold ones; y += K v; the wrap of y[2]; pose and x_pre follow y[0:3] (Robot.cpp:596-602). */
+template <int D>
+__global__ void __launch_bounds__(EKF_BLOCK) k_pose_apply(EkfGeom g, EkfBuffers b, const double2* __restrict__ K2,
+                                                          const double2* __restrict__ KS2, int max_np) {
+  EkfDevState* st = b.st;
+  const int gid = blockIdx.x * blockDim.x + threadIdx.x;
+  if (st->fix_status != EKF_FIX_ACCEPTED) {
+    if (gid == 0) st->np = 0;                                         /* nothing for the sweep: P stays bit for bit */
+    return;
+  }
+  const int nl = 3 + 2 * st->L;
+  const double v0 = st->fix_v[0], v1 = st->fix_v[1], v2 = st->fix_v[2];
+  const double2* K = b.Kp;
+  const double2* KS = b.KSp;
+  const double2 z2 = make_double2(0.0, 0.0);
+  double2 ks1[3], ks2[3];
+#pragma unroll
+  for (int r = 0; r < 3; ++r) { ks1[r] = KS[r]; ks2[r] = D == 3 ? KS2[r] : z2; }
+  for (int q = 3 + gid; q < nl; q += gridDim.x * blockDim.x) {
+    const double2 k1 = K[q], k2 = D == 3 ? K2[q] : z2;
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+      double p = sub_rank2(b.top[(size_t)r * g.ld + q], ks1[r], k1);
+      if (D == 3) p = sub_rank2(p, ks2[r], k2);
+      b.top[(size_t)r * g.ld + q] = p;
+    }
+    const double2 s1 = KS[q], s2 = D == 3 ? KS2[q] : z2;
+    const int jj = (q - 3) >> 1;
+    if (q & 1) {                                                      /* q = a: (a,a), (a,b) */
+      const double2 k1b = K[q + 1], k2b = D == 3 ? K2[q + 1] : z2;
+      double paa = sub_rank2(b.diag[4 * jj], s1, k1), pab = sub_rank2(b.diag[4 * jj + 1], s1, k1b);
+      if (D == 3) { paa = sub_rank2(paa, s2, k2); pab = sub_rank2(pab, s2, k2b); }
+      b.diag[4 * jj] = paa; b.diag[4 * jj + 1] = pab;
+    } else {                                                          /* q = b: (b,b) */
+      double pbb = sub_rank2(b.diag[4 * jj + 2], s1, k1);
+      if (D == 3) pbb = sub_rank2(pbb, s2, k2);
+      b.diag[4 * jj + 2] = pbb;
+    }
+    double t = 0.0;                                                   /* y += K v (NN) */
+    axpy_skip(t, k1.x, v0);
+    if (D > 1) axpy_skip(t, k1.y, v1);
+    if (D > 2) axpy_skip(t, k2.x, v2);
+    b.y[q] = add_rn(b.y[q], t);
+  }
+  if (gid == 0) {
+    const double2 kk1[3] = {K[0], K[1], K[2]};
+    const double2 kk2[3] = {D == 3 ? K2[0] : z2, D == 3 ? K2[1] : z2, D == 3 ? K2[2] : z2};
+    for (int r = 0; r < 3; ++r)
+      for (int q = r; q < 3; ++q) {
+        double p = sub_rank2(b.top[(size_t)r * g.ld + q], ks1[r], kk1[q]);
+        if (D == 3) p = sub_rank2(p, ks2[r], kk2[q]);
+        b.top[(size_t)r * g.ld + q] = p;
+      }
+    double yn[3];
+    for (int r = 0; r < 3; ++r) {
+      double t = 0.0;
+      axpy_skip(t, kk1[r].x, v0);
+      if (D > 1) axpy_skip(t, kk1[r].y, v1);
+      if (D > 2) axpy_skip(t, kk2[r].x, v2);
+      yn[r] = add_rn(b.y[r], t);
+    }
+    normalize_radian(yn[2]);
+    for (int r = 0; r < 3; ++r) { b.y[r] = yn[r]; st->pose[r] = yn[r]; st->x_pre[r] = yn[r]; }
+    st->np = min(max_np, D == 3 ? 2 : 1);
+  }
+}
+
+/* one pending slot only: term 2 moves into slot 0 for a second one-term sweep */
+__global__ void __launch_bounds__(EKF_BLOCK) k_pose_term2(EkfGeom g, EkfBuffers b, int d, const double2* __restrict__ K2,
+                                                          const double2* __restrict__ KS2) {
+  const bool on = d == 3 && b.st->fix_status == EKF_FIX_ACCEPTED;
+  const int gid = blockIdx.x * blockDim.x + threadIdx.x;
+  if (gid == 0) b.st->np = on ? 1 : 0;
+  if (!on) return;
+  const int nl = 3 + 2 * b.st->L;
+  for (int r = gid; r < nl; r += gridDim.x * blockDim.x) { b.Kp[r] = K2[r]; b.KSp[r] = KS2[r]; }
+}
+
 inline int blocks_for(long long n, int cap = 1 << 20) {
   long long bl = (n + EKF_BLOCK - 1) / EKF_BLOCK;
   if (bl < 1) bl = 1;
@@ -2187,6 +2345,29 @@ cudaError_t ekf_launch_remove_cold(const double* src, size_t ld_src, int src_row
   if (nr <= 0) return cudaSuccess;
   if (keep) k_remove_cold<true><<<nr, EKF_BLOCK, 0, s>>>(src, ld_src, src_row0, dst, ld_dst, dst_row0, keep, r0, nr, nl, c_from);
   else k_remove_cold<false><<<nr, EKF_BLOCK, 0, s>>>(src, ld_src, src_row0, dst, ld_dst, dst_row0, keep, r0, nr, nl, c_from);
+  return cudaGetLastError();
+}
+cudaError_t ekf_launch_pose_gain(const EkfGeom& g, const EkfBuffers& b, const EkfPoseFix& f, int d, double2* K2,
+                                 double2* KS2, int L_ub, cudaStream_t s) {
+  const int grid = blocks_for(3 + 2LL * L_ub, 148 * 8);
+  if (d == 1) k_pose_gain<1><<<grid, EKF_BLOCK, 0, s>>>(g, b, f, K2, KS2);
+  else if (d == 2) k_pose_gain<2><<<grid, EKF_BLOCK, 0, s>>>(g, b, f, K2, KS2);
+  else if (d == 3) k_pose_gain<3><<<grid, EKF_BLOCK, 0, s>>>(g, b, f, K2, KS2);
+  else return cudaErrorInvalidValue;
+  return cudaGetLastError();
+}
+cudaError_t ekf_launch_pose_apply(const EkfGeom& g, const EkfBuffers& b, int d, const double2* K2, const double2* KS2,
+                                  int max_np, int L_ub, cudaStream_t s) {
+  const int grid = blocks_for(2LL * L_ub + 1, 148 * 8);
+  if (d == 1) k_pose_apply<1><<<grid, EKF_BLOCK, 0, s>>>(g, b, K2, KS2, max_np);
+  else if (d == 2) k_pose_apply<2><<<grid, EKF_BLOCK, 0, s>>>(g, b, K2, KS2, max_np);
+  else if (d == 3) k_pose_apply<3><<<grid, EKF_BLOCK, 0, s>>>(g, b, K2, KS2, max_np);
+  else return cudaErrorInvalidValue;
+  return cudaGetLastError();
+}
+cudaError_t ekf_launch_pose_term2(const EkfGeom& g, const EkfBuffers& b, int d, const double2* K2, const double2* KS2,
+                                  int L_ub, cudaStream_t s) {
+  k_pose_term2<<<blocks_for(3 + 2LL * L_ub, 148 * 8), EKF_BLOCK, 0, s>>>(g, b, d, K2, KS2);
   return cudaGetLastError();
 }
 cudaError_t ekf_launch_zero_pending(const EkfGeom& g, const EkfBuffers& b, int m, int* d_np, cudaStream_t s) {

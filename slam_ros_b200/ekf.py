@@ -18,6 +18,7 @@ EKF_FLAG_SWEEP_DIRECT = 2
 EKF_FLAG_PER_LINE_KERNELS = 4
 EKF_FLAG_NO_OVERLAP = 8
 EKF_FLAG_FULL_GATES = 16
+EKF_POSE_X, EKF_POSE_Y, EKF_POSE_THETA = 1, 2, 4
 _STATUS = {0: "OK", 1: "EINVAL", 2: "ECAPACITY", 3: "ESINGULAR", 4: "ECUDA", 5: "ENCCL", 6: "ENOMEM", 7: "ESTATE"}
 
 _dp = C.POINTER(C.c_double)
@@ -44,7 +45,8 @@ def library_path():
 SYMBOLS = [
     "ekf_default_config", "ekf_create", "ekf_destroy", "ekf_last_error", "ekf_predict", "ekf_associate",
     "ekf_update", "ekf_add_line", "ekf_end_scan", "ekf_scan", "ekf_scan_device", "ekf_sync", "ekf_get_state",
-    "ekf_get_robot_cov", "ekf_get_ellipse", "ekf_download", "ekf_upload", "ekf_remove_lines", "ekf_download_live",
+    "ekf_get_robot_cov", "ekf_get_ellipse", "ekf_download", "ekf_upload", "ekf_remove_lines", "ekf_observe_pose",
+    "ekf_download_live",
     "ekf_download_block", "ekf_cov_stats", "ekf_profile_enable", "ekf_profile_read", "ekf_profile_read_lines", "ekf_timer_start", "ekf_timer_stop", "ekf_sweep_probe",
     "ekf_nccl_unique_id", "ekf_create_sharded", "ekf_shard_ipc_handle", "ekf_shard_connect", "ekf_shard_use_fused", "ekf_batch_create", "ekf_batch_destroy", "ekf_batch_scan",
     "ekf_batch_submit", "ekf_batch_collect", "ekf_batch_scan_device", "ekf_batch_sync", "ekf_batch_download", "ekf_batch_last_error", "ekf_version",
@@ -89,6 +91,7 @@ def load_library():
     lib.ekf_download.argtypes = [vp, _dp, _dp, _ip]
     lib.ekf_upload.argtypes = [vp, _dp, _dp, C.c_int]
     lib.ekf_remove_lines.argtypes = [vp, C.c_int, _ip, _ip]
+    lib.ekf_observe_pose.argtypes = [vp, C.c_int, _dp, _dp, C.c_double, _dp, _ip, _dp]
     lib.ekf_download_live.argtypes = [vp, _dp, _dp, C.c_int, C.c_int, _ip]
     lib.ekf_download_block.argtypes = [vp, C.c_int, C.c_int, C.c_int, C.c_int, _dp]
     lib.ekf_cov_stats.argtypes = [vp, _dp, _dp, _dp]
@@ -314,6 +317,16 @@ class EkfFilter:
         self._check(self._lib.ekf_remove_lines(self._h, idx.size, idx.ctypes.data_as(_ip) if idx.size else None,
                                                C.byref(L)), "ekf_remove_lines")
         return int(L.value)
+
+    def observe_pose(self, z, R, mask=7, d2_max=float("inf")):
+        """Fuses an absolute measurement of the components `mask` selects (EKF_POSE_X | EKF_POSE_Y | EKF_POSE_THETA) of
+        the pose: z = (x, y, theta), R = its 3x3 covariance (only the selected entries are read).  The fix is accepted
+        iff S is nonsingular and d2 <= d2_max.  Returns (status, accepted, d2, pose): status EKF_OK, or EKF_ESINGULAR for
+        a singular S (state unchanged); pose = the resulting xPos, yPos, thetaPos."""
+        za = _arr(z, (3,)); Ra = _arr(R, (9,)); d2 = C.c_double(0); acc = C.c_int(0); pose = np.zeros(3)
+        rc = self._check(self._lib.ekf_observe_pose(self._h, int(mask), _p(za), _p(Ra), float(d2_max), C.byref(d2),
+                                                    C.byref(acc), _p(pose)), "ekf_observe_pose", allow=(EKF_ESINGULAR,))
+        return rc, bool(acc.value), float(d2.value), pose
 
     def cov_stats(self):
         t = C.c_double(0); s = C.c_double(0); q = C.c_double(0)

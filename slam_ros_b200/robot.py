@@ -122,6 +122,16 @@ class Robot:
         Returns the new savedLineCount."""
         return self._f.remove_lines(indices)
 
+    def observe_pose(self, z, R, mask=7, d2_max=float("inf")):
+        """Not in the reference: fuses an absolute pose measurement (ekf_observe_pose; z = (x, y, theta), R its 3x3
+        covariance, mask of EKF_POSE_X | EKF_POSE_Y | EKF_POSE_THETA).  The pose mirrors xPos / yPos / thetaPos follow
+        the corrected pose: `localize` passes them as x_t0 (Robot.cpp:130), so a stale mirror would overwrite the fix at
+        the next prediction.  As after any update, the next `localize` forms its odometry from the corrected pose and
+        the encoder pose (Robot.cpp:140-145, SURVEY Q5).  Returns (status, accepted, d2)."""
+        rc, acc, d2, pose = self._f.observe_pose(z, R, mask=mask, d2_max=d2_max)
+        self.xPos, self.yPos, self.thetaPos = float(pose[0]), float(pose[1]), float(pose[2])
+        return rc, acc, d2
+
     def getEllipse(self):
         """Robot::getEllipse (Robot.cpp:73-124) -> (ok, (axis0, axis1), angle)."""
         return self._f.get_ellipse()
