@@ -114,7 +114,17 @@ int ekf_sync(ekf_ctx* ctx);
 /* --- state access -------------------------------------------------------------------------------- */
 
 /* xPos/yPos/thetaPos, savedLineCount and the sticky status (EKF_ECAPACITY / EKF_ESINGULAR seen since
- * the last call; cleared by the call).  Any pointer may be NULL. */
+ * the last call; cleared by the call).  Any pointer may be NULL.
+ *
+ * Status of a scan.  EKF_ECAPACITY: more unmatched lines than free slots; the first ones in line order were appended,
+ * the rest dropped (then the reset policy applies as usual).  EKF_ESINGULAR: the first fit of some line skipped a
+ * pair whose S has a zero pivot in its LU before the landmark it matched (or anywhere, if it matched nothing); the
+ * search went on past it.  A singular pair past a line's match is not reported, on any path.  When a scan hits both,
+ * EKF_ECAPACITY is reported.
+ * Every scan ORs its status into a sticky word on the device.  ekf_scan and ekf_end_scan return it and clear it, so
+ * they report their own scan plus any ekf_scan_device scan not read yet, and the next clean scan returns EKF_OK.
+ * ekf_scan_device reports nothing: ekf_get_state with sticky_status != NULL waits for the scans enqueued before it,
+ * returns the word (ECAPACITY first) and clears it; with sticky_status == NULL it leaves the word as it is. */
 int ekf_get_state(ekf_ctx* ctx, double pose[3], int* n_lines, int* sticky_status);
 
 /* P_t0[0:3,0:3] row-major, symmetrised: what Robot::getEllipse reads (Robot.cpp:75-77). */
@@ -221,12 +231,18 @@ int ekf_shard_use_fused(ekf_ctx* ctx, int on);
 typedef struct ekf_batch ekf_batch;
 int ekf_batch_create(ekf_batch** out, const ekf_config* cfg, int n_filters);
 int ekf_batch_destroy(ekf_batch* b);
-/* One localize per filter.  u: B x 3, z: B x m x 2, R: B x m x 4, j_out (nullable): B x m, pose (nullable): B x 3. */
+/* One localize per filter.  u: B x 3, z: B x m x 2, R: B x m x 4, j_out (nullable): B x m, pose (nullable): B x 3.
+ * Status: of this step alone, over all filters: EKF_ECAPACITY if a filter dropped a line, else EKF_ESINGULAR if a
+ * filter's first fit skipped a singular pair before its match (as for ekf_get_state).  One exception: without
+ * EKF_FLAG_FULL_GATES a landmark with S00 > 0 whose angle innovation alone puts it beyond twice the gate is not gated
+ * in full, so a singular S of that pair goes unreported (the association is the same: it is no match either way); a
+ * pair with S00 == 0 is always gated. */
 int ekf_batch_scan(ekf_batch* b, const double* u, int m, const double* z, const double* R, int* j_out,
                    double* pose);
 /* The same, pipelined: ekf_batch_submit stages the step's inputs and returns at once (at most two steps in flight: the
  * inputs of step s+1 are copied while the kernel of step s runs); ekf_batch_collect waits for the OLDEST submitted step
- * and returns its matches, poses and status.  ekf_batch_scan == submit + collect. */
+ * and returns its matches, poses and status: the status of that step, not of the one submitted after it.
+ * ekf_batch_scan == submit + collect.  ekf_batch_scan_device reports no status. */
 int ekf_batch_submit(ekf_batch* b, const double* u, int m, const double* z, const double* R);
 int ekf_batch_collect(ekf_batch* b, int* j_out, double* pose);
 int ekf_batch_scan_device(ekf_batch* b, const double* d_u, int m, const double* d_z, const double* d_R,

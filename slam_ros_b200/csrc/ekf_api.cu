@@ -107,7 +107,7 @@ struct ekf_ctx {
   unsigned long long* d_counters;   /* tile counters of the sweep passes: [0,16) line stream, [16,32) sweep stream */
   cudaEvent_t evE, evF[2];
   int evF_used[2];
-  struct { int *jbest, *jout, *pidx, *eidx, *ext; double* ext_cs; } tab[2];
+  struct { int *jbest, *jsing, *jout, *pidx, *eidx, *ext; double* ext_cs; } tab[2];
   int num_sms;
   int cluster;         /* CTAs in the line-loop cluster */
   int sweep_shape;     /* 0: 64x64 tiles, 1: 32x128, 2: 16x256 (EKF_SWEEP_SHAPE) */
@@ -171,19 +171,19 @@ double* in_z(ekf_ctx* c) { return c->d_in + 6; }
 double* in_R(ekf_ctx* c) { return c->d_in + 6 + 2 * (size_t)c->max_lines; }
 
 void use_tables(ekf_ctx* ctx, int t) {
-  ctx->b.jbest = ctx->tab[t].jbest; ctx->b.jout = ctx->tab[t].jout; ctx->b.pidx = ctx->tab[t].pidx;
+  ctx->b.jbest = ctx->tab[t].jbest; ctx->b.jsing = ctx->tab[t].jsing; ctx->b.jout = ctx->tab[t].jout; ctx->b.pidx = ctx->tab[t].pidx;
   ctx->b.eidx = ctx->tab[t].eidx; ctx->b.ext = ctx->tab[t].ext; ctx->b.ext_cs = ctx->tab[t].ext_cs;
 }
 
 int free_line_tables(ekf_ctx* ctx) {
   for (int t = 0; t < 2; ++t) {
-    cudaFree(ctx->tab[t].jbest); cudaFree(ctx->tab[t].jout); cudaFree(ctx->tab[t].pidx); cudaFree(ctx->tab[t].eidx);
+    cudaFree(ctx->tab[t].jbest); cudaFree(ctx->tab[t].jsing); cudaFree(ctx->tab[t].jout); cudaFree(ctx->tab[t].pidx); cudaFree(ctx->tab[t].eidx);
     cudaFree(ctx->tab[t].ext); cudaFree(ctx->tab[t].ext_cs);
     memset(&ctx->tab[t], 0, sizeof ctx->tab[t]);
   }
   cudaFree(ctx->d_in);
   cudaFreeHost(ctx->h_in); cudaFreeHost(ctx->h_jout);
-  ctx->b.jbest = ctx->b.jout = ctx->b.pidx = ctx->b.eidx = ctx->b.ext = 0; ctx->b.ext_cs = 0; ctx->d_in = 0;
+  ctx->b.jbest = ctx->b.jsing = ctx->b.jout = ctx->b.pidx = ctx->b.eidx = ctx->b.ext = 0; ctx->b.ext_cs = 0; ctx->d_in = 0;
   ctx->h_in = 0; ctx->h_jout = 0;
   return 0;
 }
@@ -207,6 +207,7 @@ int ensure_lines(ekf_ctx* ctx, int m) {
   const size_t n1 = (size_t)cap + 1;
   for (int t = 0; t < 2; ++t) {
     CU(cudaMalloc(&ctx->tab[t].jbest, n1 * sizeof(int)));
+    CU(cudaMalloc(&ctx->tab[t].jsing, n1 * sizeof(int)));
     CU(cudaMalloc(&ctx->tab[t].jout, n1 * sizeof(int)));
     CU(cudaMalloc(&ctx->tab[t].pidx, n1 * sizeof(int)));
     CU(cudaMalloc(&ctx->tab[t].eidx, n1 * sizeof(int)));
@@ -1011,6 +1012,7 @@ int ekf_associate(ekf_ctx* ctx, const double z[2], const double R[4], int* j_out
   const int none = EKF_NO_MATCH;
   ctx->h_jout[0] = none;
   CU(cudaMemcpyAsync(ctx->b.jbest + i, ctx->h_jout, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+  CU(cudaMemcpyAsync(ctx->b.jsing + i, ctx->h_jout, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
   CU(ekf_launch_associate(ctx->g, ctx->b, in_z(ctx), in_R(ctx), i, ctx->L_ub, ctx->stream));
   if (ctx->L_ub > 0) {
     CU(ekf_launch_gain(ctx->g, ctx->b, in_z(ctx), in_R(ctx), i, -1, 3, 1, ctx->cfg.max_batch, ctx->stream));

@@ -406,7 +406,7 @@ __device__ __forceinline__ void batch_scan_body(const EkfBatchGeom& g, const int
       const double Rl[4] = {Rs[4 * i], Rs[4 * i + 1], Rs[4 * i + 2], Rs[4 * i + 3]};
       const double xp[3] = {s_xpre[0], s_xpre[1], s_xpre[2]};
       const double P22 = Ps[tri(2) + 2];
-      int best = EKF_NO_MATCH;
+      int best = EKF_NO_MATCH, sing = EKF_NO_MATCH;                   /* sing: this lane's lowest singular pair */
       int j0 = 0;
       while (j0 < L && best == EKF_NO_MATCH) {                        /* first fit: a match among these candidates ends the search */
         /* rounds of 32 landmarks take the pre-test; their survivors, in index order, fill the lanes of ONE round of full
@@ -463,7 +463,7 @@ __device__ __forceinline__ void batch_scan_body(const EkfBatchGeom& g, const int
           Cm[3][3] = ca_[a]; Cm[3][4] = Cm[4][3] = cb_[a]; Cm[4][4] = cb_[bb];
           BT_MARK(13);
           gate_from_block(Cm, ys[a], ys[bb], xp, z0, z1, Rl, Gj);
-          if (Gj.singular) atomicOr(&s_sticky, EKF_STICKY_SINGULAR);
+          if (Gj.singular) sing = min(sing, jj);
           else if (!gate_rejects_d2(Gj.d2, g.gate_d2max)) mine = jj;                   /* :489 */
           BT_MARK(14);
         }
@@ -471,7 +471,10 @@ __device__ __forceinline__ void batch_scan_body(const EkfBatchGeom& g, const int
         if (mine != EKF_NO_MATCH && mine == best) sG = Gj;            /* the winner publishes its gate record */
         BT_MARK(15);
       }
+      /* EKF_ESINGULAR: a singular pair that first fit skipped before its winner (any, when the line matched nothing) */
+      sing = __reduce_min_sync(0xffffffffu, sing);
       if (lane == 0) {
+        if (sing < best) atomicOr(&s_sticky, EKF_STICKY_SINGULAR);
         s_best = best;
         if (best == EKF_NO_MATCH) { ext[ne] = i; if (jout) jout[i] = -1; }           /* :309 / :325 / :493 */
         else { matched[best] = 1; if (jout) jout[i] = best; }                       /* :501 */

@@ -90,6 +90,7 @@ struct EkfBuffers {
   double* colB;
   /* per-scan line tables, sized max_lines (+1 for the prefix counters) */
   int* jbest;         /* first-fit winner per line (EKF_NO_MATCH = none) */
+  int* jsing;         /* lowest landmark whose pair with the line has a singular S (EKF_NO_MATCH = none) */
   int* jout;          /* matched landmark or -1 per line */
   int* pidx;          /* pidx[i] = matches before line i; pidx[m] = matches in the scan */
   int* eidx;          /* eidx[i] = unmatched lines before line i */

@@ -106,7 +106,7 @@ __device__ __forceinline__ void predict_body(const EkfGeom& g, const EkfBuffers&
     r1.x = add_rn(0.0, r1.x); axpy_skip(r1.x, F12, p2.x); r1.y = add_rn(0.0, r1.y); axpy_skip(r1.y, F12, p2.y);
     *reinterpret_cast<double2*>(t0p + q) = r0; *reinterpret_cast<double2*>(t1p + q) = r1;
   }
-  for (int i = gid; i < m; i += stride) { b.jbest[i] = EKF_NO_MATCH; b.jout[i] = -1; }
+  for (int i = gid; i < m; i += stride) { b.jbest[i] = EKF_NO_MATCH; b.jsing[i] = EKF_NO_MATCH; b.jout[i] = -1; }
   if (gid == 0) {
     double A[3][3], T[3][3], Pn[3][3];
     load_rr(g, b.top, A);
@@ -167,7 +167,7 @@ __global__ void __launch_bounds__(EKF_BLOCK) k_associate(EkfGeom g, EkfBuffers b
     const double Rl[4] = {R[4 * line], R[4 * line + 1], R[4 * line + 2], R[4 * line + 3]};
     Gate G;
     eval_gate(g, b, xp, j, z[2 * line], z[2 * line + 1], Rl, G);
-    if (G.singular) atomicOr(&b.st->sticky, EKF_STICKY_SINGULAR);
+    if (G.singular) atomicMin(&b.jsing[line], j);                   /* reported by k_end_scan_a if below the winner */
     else if (!gate_rejects_d2(G.d2, g.gate_d2max)) cand = j;          /* :489 */
   }
   cand = __reduce_min_sync(0xffffffffu, cand);
@@ -546,7 +546,7 @@ __global__ void __launch_bounds__(FL_THREADS, FL_THREADS == 256 ? 3 : 1) k_scan_
         Cm[3][3] = daa; Cm[3][4] = Cm[4][3] = dab; Cm[4][4] = dbb;
         Gate G;
         gate_from_block(Cm, ya, yb, xp, z0, z1, Rl, G);
-        if (G.singular) atomicOr(&st->sticky, EKF_STICKY_SINGULAR);
+        if (G.singular) atomicMin(&b.jsing[line], j);                 /* reported by k_end_scan_a if below the winner */
         else if (!gate_rejects_d2(G.d2, g.gate_d2max)) { cand = j; gate_store(b.gates + (size_t)GATE_REC * j, G); }
       }
     }
@@ -768,7 +768,7 @@ __global__ void __launch_bounds__(FL_THREADS, 1) k_scan_lines2(EkfGeom g, EkfBuf
         Cm[3][3] = h.daa; Cm[3][4] = Cm[4][3] = h.dab; Cm[4][4] = h.dbb;
         Gate G;
         gate_from_block(Cm, h.ya, h.yb, xp, z0, z1, Rl, G);
-        if (G.singular) atomicOr(&st->sticky, EKF_STICKY_SINGULAR);
+        if (G.singular) atomicMin(&b.jsing[line], j);                 /* reported by k_end_scan_a if below the winner */
         else if (!gate_rejects_d2(G.d2, g.gate_d2max)) {
           cand = j;
           double* rec = b.gates + (size_t)GATE_REC * j;
@@ -1562,6 +1562,11 @@ __global__ void __launch_bounds__(512) k_end_scan_a(EkfGeom g, EkfBuffers b, con
   if (threadIdx.x == 0 && blockIdx.x == 0) {
     st->n_added = n_add;
     if (n_add < ne) atomicOr(&st->sticky, EKF_STICKY_CAPACITY);       /* the reference overruns y[] here (Q4) */
+  }
+  {     /* EKF_ESINGULAR: some line's first fit skipped a singular pair before its winner (any, when it matched nothing) */
+    int skipped = 0;
+    for (int i = threadIdx.x; i < m; i += blockDim.x) skipped |= b.jsing[i] < b.jbest[i];
+    if (__syncthreads_or(skipped) && threadIdx.x == 0) atomicOr(&st->sticky, EKF_STICKY_SINGULAR);
   }
   /* this scan's pending terms have no entry for the rows being appended: zero them, so that the (possibly
    * later) sweep and the next scan's on-the-fly corrections see K = 0 there */

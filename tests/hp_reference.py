@@ -244,6 +244,7 @@ class HPFilter:
         self.matched = set()
         self.extra = []
         self.matches = 0
+        self.singular = False        # a pair with singular S was skipped in this scan
         self.depth += DEPTH_PREDICT
 
     # ---- Robot.cpp:367-489 for every unmatched landmark at once --------------------------------------------
@@ -271,8 +272,9 @@ class HPFilter:
         S = H @ C5 @ np.swapaxes(H, 1, 2) + Rm.astype(LD)
         det = S[:, 0, 0] * S[:, 1, 1] - S[:, 0, 1] * S[:, 1, 0]
         Si = np.empty_like(S)
-        Si[:, 0, 0] = S[:, 1, 1] / det; Si[:, 1, 1] = S[:, 0, 0] / det
-        Si[:, 0, 1] = -S[:, 0, 1] / det; Si[:, 1, 0] = -S[:, 1, 0] / det
+        with np.errstate(divide="ignore", invalid="ignore"):             # det == 0: a singular pair, skipped
+            Si[:, 0, 0] = S[:, 1, 1] / det; Si[:, 1, 1] = S[:, 0, 0] / det
+            Si[:, 0, 1] = -S[:, 0, 1] / det; Si[:, 1, 0] = -S[:, 1, 0] / det
         z = np.asarray(z, np.float64).astype(LD)
         h0, cw = normalize_radians(y[a] - xp[2])
         mh0 = _f(y[a]) + _f(xp[2]) + cw
@@ -285,7 +287,8 @@ class HPFilter:
         up = ~dn & (np.abs(v0 + TWO_PI) < np.abs(v0))
         v0 = np.where(dn, v0 - TWO_PI, np.where(up, v0 + TWO_PI, v0))
         mv0 = mv0 + np.where(dn | up, float(TWO_PI), 0.0)
-        d2 = v0 * (Si[:, 0, 0] * v0 + Si[:, 1, 0] * v1) + v1 * (Si[:, 0, 1] * v0 + Si[:, 1, 1] * v1)
+        with np.errstate(invalid="ignore"):
+            d2 = v0 * (Si[:, 0, 0] * v0 + Si[:, 1, 0] * v1) + v1 * (Si[:, 0, 1] * v0 + Si[:, 1, 1] * v1)
         rec = dict(js=js, c=c, s=s, g=g, S=S, Si=Si, v=np.stack([v0, v1], 1),
                    mv=np.stack([mv0, mv1], 1), det=det)
         return js, d2, rec
@@ -294,7 +297,8 @@ class HPFilter:
         js, d2, rec = self.gates(z, R)
         gate = LD(self.gate)
         for i in range(js.size):
-            if rec["det"][i] == 0:
+            if rec["det"][i] == 0:                 # singular S: the pair is no match, EKF_ESINGULAR (ekf.h)
+                self.singular = True
                 continue
             d = np.sqrt(abs(d2[i]))
             if math.isfinite(self.gate) and self.gate > 0:
@@ -393,10 +397,13 @@ class HPFilter:
             self.T[:, 3:] = 0; self.mT[:, 3:] = 0
             self.base = np.zeros((0, 0)); self.aug = {}
             self._clear_terms()
+        if status == 0 and self.singular:                              # EKF_ECAPACITY takes precedence
+            status = 3
         return status
 
     def scan(self, u, z, R):
-        """One Robot::localize with odometry u.  Returns (status, j_out)."""
+        """One Robot::localize with odometry u.  Returns (status, j_out): status 0, 2 (a line did not fit: EKF_ECAPACITY)
+        or 3 (the first fit of some line skipped a pair with singular S: EKF_ESINGULAR)."""
         z = np.asarray(z, np.float64).reshape(-1, 2); R = np.asarray(R, np.float64).reshape(-1, 4)
         m = z.shape[0]
         self.predict(u)
