@@ -56,7 +56,12 @@ typedef struct {
   double encoder_noise; /* ENCODERNOISE        (Robot.h:17, 0.024) */
   int reset_headroom;   /* the 10 of "savedLineCount > LINESIZE-10" (Robot.cpp:893) */
   int device;           /* CUDA device ordinal */
-  int max_batch;        /* most matched lines folded into one deferred sweep (default 64) */
+  int max_batch;        /* most lines folded into one deferred in-place sweep (default 64; <= 0 means 64).  It counts
+                           lines on the scan paths (matched or not) and ekf_update calls on the step-wise path.  It also
+                           sizes the overlapped pipeline: below 16 nothing overlaps; from 16 to 63 the slot ring halves
+                           hold max_batch / 2 (at most 32) terms, and scans of more lines than that, up to 32, run in
+                           place; from 64 on they hold 64.  Above 64 the fused line loop is off: in-place scans run the
+                           per-line kernels.  Every value gives the same results, bit for bit. */
   int flags;            /* EKF_FLAG_* */
 } ekf_config;
 

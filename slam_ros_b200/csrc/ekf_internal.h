@@ -9,8 +9,9 @@
  *   P     [rows][ld]      every other ("cold") element, UPPER triangle authoritative, row-major,
  *                         64-row tile rows; in the row-sharded mode a rank stores only the tile rows
  *                         rb with rb % world == rank (local row = (rb / world) * 64 + r % 64)
- *   Kp,KSp[max_batch][ld] double2: the scan's pending gains K_i and K_i*S_i (rank-2 terms not yet
- *                         folded into the cold part)
+ *   Kp,KSp[slots][ld]     double2: the scan's pending gains K_i and K_i*S_i (rank-2 terms not yet
+ *                         folded into the cold part); slots = max(max_batch, 2 * group), the overlapped
+ *                         path's ring of two halves of `group` slots (ekf_api.cu, create_common)
  *
  * Hot elements are kept current after every matched line (O(n) work); the cold part is brought up
  * to date by ONE sweep per scan -- or per group of scans on the overlapped path -- that applies the

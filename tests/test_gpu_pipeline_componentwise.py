@@ -129,17 +129,22 @@ def case_inputs(name):
 
 
 # ---- the intended grouping (the host rules of DESIGN section 5) -------------------------------------------------------
-def knobs(env):
-    """The host's sizing of the slot ring and the group budget (ekf_api.cu, create_common), at the default max_batch = 64:
-    group = 64, capped at 2 x ekf_sweep_terms_per_pass(shape, 64), which is min(32, EKF_SWEEP_MAXC) for the sweep shapes
+def knobs(env, max_batch=64):
+    """The host's sizing of the slot ring and the group budget (ekf_api.cu, create_common) for ekf_config.max_batch:
+    group = 64 from max_batch = 64 on, else min(max_batch / 2, 32); slots (rows of Kp / KSp) = max(max_batch, 2 group);
+    then group capped at 2 x ekf_sweep_terms_per_pass(shape, 64), which is min(32, EKF_SWEEP_MAXC) for the sweep shapes
     the variants use (0, 10, 11); budget = min(EKF_SWEEP_GROUP or 16, group); chunks of min(16, group) lines above 32.
-    If that sizing changes (per shape, or with max_batch), update this function: the grouping assertions depend on it."""
+    Below max_batch = 16 nothing overlaps.  If that sizing changes, update this function: the grouping assertions
+    depend on it."""
+    mb = max_batch if max_batch > 0 else 64
     maxc = int(env.get("EKF_SWEEP_MAXC", 32))
     maxc = maxc if maxc in (8, 16, 32) else 32
-    group = min(64, 2 * min(32, maxc))          # ring half: 2 x ekf_sweep_terms_per_pass(shape 0/9/10/11, 64)
+    group = 64 if mb >= 64 else min(mb // 2, 32)
+    slots = max(mb, 2 * group)
+    group = max(1, min(group, 2 * min(32, maxc)))   # ring half: 2 x ekf_sweep_terms_per_pass(shape 0/9/10/11, 64)
     budget = max(0, min(int(env.get("EKF_SWEEP_GROUP", 16)), group))
-    return dict(group=group, budget=budget, chunk=min(16, group), chunk_above=32,
-                line_sms=int(env.get("EKF_LINE_SMS", -1)))
+    return dict(group=group, slots=slots, budget=budget, chunk=min(16, group), chunk_above=32, max_batch=mb,
+                overlap=mb >= 16, line_sms=int(env.get("EKF_LINE_SMS", -1)))
 
 
 def line_sms(m, cap, k):
@@ -149,22 +154,40 @@ def line_sms(m, cap, k):
     return need if (m > 8 and 20 < need <= 28) else 20
 
 
-def intended_grouping(ms, cap, env):
-    """(term bound of every sweep hand-off, scans of every hand-off) for scans of ms lines on a map that stays on the
-    overlapped path, with a sync at the end.  A scan of 0 lines (or more than the ring half and unchunked) drains."""
-    k = knobs(env)
+def inplace_bounds(m, max_batch):
+    """Term bounds of the in-place sweeps of one scan of m lines on a non-empty map: the fused line loop (max_batch <= 64)
+    and the per-line kernels both fold every max_batch lines and at the end of the scan."""
+    return [min(max_batch, m - l0) for l0 in range(0, m, max_batch)]
+
+
+def intended_grouping(ms, cap, env, max_batch=64, halves=None):
+    """(term bound of every sweep, scans of every sweep) for scans of ms lines on a map that stays on the overlapped
+    path, with a sync at the end.  A scan of 0 lines, or of more than the ring half and unchunked, drains and runs in
+    place: one sweep per max_batch lines.  `halves`, if a list, receives the slot-ring half of every sweep (0 or 1; None
+    for an in-place sweep): the ring starts at half 0 when the filter is created and alternates at every hand-off."""
+    k = knobs(env, max_batch)
     bounds, members = [], []
     cur = None                                   # [term bound, line-loop SMs, scans] of the open group
+    par = [0]
+
+    def add(bound, scans, ring=True):
+        bounds.append(bound); members.append(scans)
+        if halves is not None:
+            halves.append(par[0] if ring else None)
+        if ring:
+            par[0] ^= 1
 
     def close():
         nonlocal cur
         if cur is not None:
-            bounds.append(cur[0]); members.append(cur[2]); cur = None
+            add(cur[0], cur[2]); cur = None
 
     for s, m in enumerate(ms):
         chunked = k["chunk"] > 0 and m > k["chunk_above"]
         if m < 1 or (m > k["group"] and not chunked):
             close()
+            for b in inplace_bounds(m, k["max_batch"]):
+                add(b, [s], ring=False)
             continue
         ls = line_sms(m, cap, k)
         groupable = k["budget"] > 0 and not chunked
@@ -174,7 +197,7 @@ def intended_grouping(ms, cap, env):
         if not groupable:
             step = k["chunk"] if chunked else m
             for l0 in range(0, m, step):
-                bounds.append(min(step, m - l0)); members.append([s])
+                add(min(step, m - l0), [s])
             continue
         if cur is None:
             cur = [0, ls, []]
@@ -249,12 +272,13 @@ def reference(name):
 
 
 # ---- device side (runs in a subprocess, with the environment under test) --------------------------------------------
-def device_run(name, blocks, out_path):
+def device_run(name, blocks, out_path, cfg=None):
+    """cfg: further ekf_config fields (max_batch, flags) of the filter under test."""
     from slam_ros_b200 import EkfFilter
     c = case_inputs(name)
     spec = CASES[name]
     res = {}
-    f = EkfFilter(capacity_lines=c["cap"], reset_headroom=c["headroom"])
+    f = EkfFilter(capacity_lines=c["cap"], reset_headroom=c["headroom"], **(cfg or {}))
     if "warm" in c:
         wy, wP, wL, wscans = c["warm"]
         f.upload(wy, wP, wL)
@@ -297,12 +321,15 @@ def device_run(name, blocks, out_path):
     np.savez(out_path, **res)
 
 
-def _spawn(name, env_extra, workdir, lib=None):
-    """device_run(name) in a child process with the environment under test; its results go to a file in workdir."""
+def _spawn(name, env_extra, workdir, lib=None, cfg=None, module=None):
+    """device_run(name, cfg) in a child process with the environment under test; its results go to a file in workdir.
+    module: a test module to import first in the child (one that adds its own cases to CASES)."""
     ref = reference(name)
-    path = os.path.join(str(workdir), "%s_%s.npz" % (name, abs(hash(json.dumps(env_extra, sort_keys=True) + str(lib)))))
-    code = ("import sys; sys.path[:0] = [%r, %r]\nimport test_gpu_pipeline_componentwise as t\n"
-            "t.device_run(%r, %r, %r)\n" % (ROOT, TESTS, name, [list(b) for b in ref["blocks"]], path))
+    key = json.dumps([env_extra, cfg], sort_keys=True) + str(lib)
+    path = os.path.join(str(workdir), "%s_%s.npz" % (name, abs(hash(key))))
+    code = ("import sys; sys.path[:0] = [%r, %r]\n%simport test_gpu_pipeline_componentwise as t\n"
+            "t.device_run(%r, %r, %r, %r)\n" % (ROOT, TESTS, ("import %s\n" % module) if module else "", name,
+                                                  [list(b) for b in ref["blocks"]], path, cfg))
     env = dict(os.environ)
     for k in ("EKF_SWEEP_GROUP", "EKF_SWEEP_MAXC", "EKF_SWEEP_SHAPE", "EKF_LINE_LOOP", "EKF_LINE_SMS", "EKF_FUSE_PREDICT",
               "EKF_LIB", "EKF_CHUNK", "EKF_CHUNK_ABOVE", "EKF_LINE_THREADS"):
@@ -357,14 +384,14 @@ def compare(dev, name):
     return worst, fails
 
 
-def check_exercised(dev, name, env, label):
+def check_exercised(dev, name, env, label, max_batch=64):
     """The case ran the path it is meant to: sweep launches and folded terms of the intended grouping, and the scan
     pattern the case is built around (from the reference's associations, equal to the device's once compare passed)."""
     ref = reference(name)
     c = case_inputs(name)
     ms = [z.shape[0] for _, z, _ in c["scans"]]
     J = [r["j"] for r in ref["scans"]]
-    bounds, members = intended_grouping(ms, c["cap"], env)
+    bounds, members = intended_grouping(ms, c["cap"], env, max_batch)
     sweeps, sweep_bytes = dev["prof"]
     n = 3.0 + 2.0 * int(dev["L"])
     terms = (sweep_bytes - sweeps * 8.0 * n * (n + 1.0)) / (32.0 * n)
@@ -382,7 +409,7 @@ def check_exercised(dev, name, env, label):
             within += int(((J[s] >= lo) & (J[s] < hi)).sum()) if hi > lo else 0
     note = "%d sweeps, %d terms, up to %d scans per sweep, %d lines matched a landmark appended earlier in their group" % (
         len(bounds), sum(bounds), shared, within)
-    budget = knobs(env)["budget"]
+    budget = knobs(env, max_batch)["budget"]
     if budget:
         assert shared >= 2 and within >= 1, "%s: %s" % (label, note)
     if name == "groups_nl1":
@@ -483,18 +510,19 @@ def test_mutant_anchors_occur_exactly_once():
         assert case in CASES
 
 
-def build_mutant(key, workdir):
-    """Copies slam_ros_b200/csrc and include (same relative layout), applies mutant `key`, starts nvcc.  Returns
-    (process, library path)."""
+def build_mutant(key, workdir, table=None, count=1):
+    """Copies slam_ros_b200/csrc and include (same relative layout), applies mutant `key` of `table` (default MUTANTS:
+    (file, anchor, replacement, ...)) at the `count` occurrences of its anchor, starts nvcc.  Returns (process, library
+    path)."""
     from slam_ros_b200 import build as b
-    fname, anchor, repl = MUTANTS[key][:3]
+    fname, anchor, repl = (table or MUTANTS)[key][:3]
     src = os.path.join(workdir, "slam_ros_b200", "csrc")
     shutil.copytree(CSRC, src)
     shutil.copytree(os.path.join(ROOT, "include"), os.path.join(workdir, "include"))
     path = os.path.join(src, fname)
     with open(path) as fh:
         text = fh.read()
-    assert text.count(anchor) == 1, (key, anchor)
+    assert text.count(anchor) == count, (key, anchor, text.count(anchor))
     with open(path, "w") as fh:
         fh.write(text.replace(anchor, repl))
     out = os.path.join(workdir, "libekfcuda_%s.so" % key)
