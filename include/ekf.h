@@ -155,6 +155,30 @@ int ekf_upload(ekf_ctx* ctx, const double* y, const double* P, int n_lines);
  * batch filters (ekf_batch_*) have no such call. */
 int ekf_remove_lines(ekf_ctx* ctx, int k, const int* lines, int* n_lines);
 
+/* Map management, not in the reference.  Appends k known landmarks -- the walls of a floor plan, or the map of an earlier
+ * session -- as landmarks savedLineCount .. savedLineCount+k-1, in order.  lines = k x (alfa, r) in the world frame, the
+ * convention of the state's own landmarks y[3+2j], y[4+2j]; alfa is stored after normalize_radian (Robot.cpp:62-71) as
+ * the augmentation stores it (:801), r as given.  cov = NULL: surveyed, every new entry of P is zero; otherwise the
+ * 2k x 2k row-major joint covariance of the new landmarks (for example the landmark block P[3:, 3:] of an earlier
+ * session's ekf_download_live).  The cross-covariance with the robot and the existing landmarks is zero.  The result is
+ * bit for bit y' = [y, lines], P' = [[P, 0], [0, cov]]; pose, x_pre and the robot covariance are unchanged.  Waits for
+ * the sweep in flight.  *n_lines (nullable) = the new savedLineCount.  k = 0 is a no-op.
+ * A landmark with zero covariance stays fixed under every scan: its rows of P are zero, so its gain rows are zero, and a
+ * line that matches it is a pure pose measurement.  One with a prior covariance is an ordinary landmark from then on.
+ * First fit takes the lowest landmark index, so a floor plan wins over SLAM duplicates of its walls only if it is
+ * inserted on a fresh filter before the first scan, or after the duplicates are removed (ekf_remove_lines).
+ * The map reset of Robot.cpp:893-904 counts inserted landmarks like any others and drops them with the map; a caller
+ * that wants them kept re-inserts them after a reset, which it sees as the line count falling.
+ * EKF_EINVAL: k < 0, NULL lines with k > 0, a non-finite entry, a cov that is not exactly symmetric, has a non-finite
+ * entry or a negative diagonal entry (positive semi-definiteness beyond that is not checked: it would cost O(k^3)), or a
+ * row-sharded filter; EKF_ECAPACITY: savedLineCount + k > capacity_lines -- the call is all or nothing, unlike a scan's
+ * augmentation, which appends what fits; EKF_ESTATE: inside an open step-wise scan.  On error the state is unchanged.
+ * The Monte-Carlo batch filters (ekf_batch_*) have no such call.
+ * Cost (one B200, DESIGN section 3.3): writes 8 (nl_old 2k + k (2k + 1)) bytes of P at about the device-to-device copy
+ * rate plus a fixed cost: 100 surveyed walls into 10 000 landmarks 0.05 ms; with cov, the host-side check and the
+ * pageable copy of cov dominate (5.1 ms for k = 1 000). */
+int ekf_insert_lines(ekf_ctx* ctx, int k, const double* lines, const double* cov, int* n_lines);
+
 /* Absolute pose measurement, not in the reference (GNSS, UWB, motion capture, a docking fiducial, a relocaliser).
  * mask selects d = popcount(mask) components of the pose; z is a full 3-vector (x, y, theta) and R a full row-major 3x3
  * covariance, of which only the selected entries are read.  With H = the selected rows of [I_3 0]:

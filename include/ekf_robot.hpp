@@ -131,6 +131,18 @@ class Robot {
     return savedLineCount;
   }
 
+  /* Not in the reference: appends known landmarks (ekf_insert_lines) and updates savedLineCount.  lines = k x (alfa, r)
+   * in the world frame, flattened; cov = NULL for surveyed walls (fixed from then on), else the 2k x 2k row-major joint
+   * covariance of an earlier map.  Insert a floor plan before the first localize (first fit takes the lowest index), and
+   * again after a map reset drops it.  Returns the new savedLineCount; throws on bad input or when the map would exceed
+   * its capacity (nothing is inserted then). */
+  int insertLines(const std::vector<double>& lines, const double* cov = nullptr) {
+    if (lines.size() % 2) throw std::invalid_argument("libekfcuda: insertLines needs (alfa, r) pairs");
+    const int rc = ekf_insert_lines(ctx_, (int)(lines.size() / 2), lines.empty() ? 0 : lines.data(), cov, &savedLineCount);
+    if (rc != EKF_OK) throw std::runtime_error(std::string("libekfcuda: ") + ekf_last_error(ctx_));
+    return savedLineCount;
+  }
+
   /* Not in the reference: fuses an absolute pose measurement (ekf_observe_pose): z = (x, y, theta), R its row-major 3x3
    * covariance, mask of EKF_POSE_X | EKF_POSE_Y | EKF_POSE_THETA (only the selected entries are read), accepted iff S
    * is nonsingular and d2 <= d2Max.  xPos / yPos / thetaPos follow the corrected pose: localize passes them as x_t0

@@ -1292,6 +1292,86 @@ int ekf_remove_lines(ekf_ctx* ctx, int k, const int* lines, int* n_lines) {
   return EKF_OK;
 }
 
+/* Appending landmarks with no cross-covariance to the rest is y' = [y, lines], P' = [[P, 0], [0, C]]: writes of the new
+ * entries, no arithmetic.  After the drain Pbuf[rd] is the one complete covariance and every later path reads from it or
+ * from a sweep that writes every live element of its destination, so only Pbuf[rd] is written (DESIGN section 3.3). */
+int ekf_insert_lines(ekf_ctx* ctx, int k, const double* lines, const double* cov, int* n_lines) {
+  if (!ctx) return EKF_EINVAL;
+  if (k < 0 || (k > 0 && !lines)) { snprintf(ctx->err, sizeof ctx->err, "ekf_insert_lines: k = %d, lines = %p", k, (const void*)lines); return EKF_EINVAL; }
+  for (int i = 0; i < 2 * k; ++i)
+    if (!isfinite(lines[i])) { snprintf(ctx->err, sizeof ctx->err, "ekf_insert_lines: lines[%d] = %g is not finite", i, lines[i]); return EKF_EINVAL; }
+  const size_t w = 2 * (size_t)k;
+  if (cov) {
+    for (size_t i = 0; i < w; ++i)
+      if (!(cov[i * w + i] >= 0.0)) {
+        snprintf(ctx->err, sizeof ctx->err, "ekf_insert_lines: cov[%zu][%zu] = %g (need a finite, non-negative diagonal)", i, i, cov[i * w + i]);
+        return EKF_EINVAL;
+      }
+    /* the upper triangle against the lower one in 64 x 64 tiles: the transposed reads stay in cache */
+    const size_t T = 64;
+    for (size_t i0 = 0; i0 < w; i0 += T)
+      for (size_t c0 = i0; c0 < w; c0 += T)
+        for (size_t i = i0; i < i0 + T && i < w; ++i)
+          for (size_t c = c0 > i ? c0 : i; c < c0 + T && c < w; ++c)
+            if (!isfinite(cov[i * w + c]) || cov[i * w + c] != cov[c * w + i]) {
+              snprintf(ctx->err, sizeof ctx->err, "ekf_insert_lines: cov[%zu][%zu] = %g is not finite or not symmetric", i, c, cov[i * w + c]);
+              return EKF_EINVAL;
+            }
+  }
+  if (ctx->g.world > 1) {
+    snprintf(ctx->err, sizeof ctx->err, "ekf_insert_lines: not supported on a row-sharded filter");
+    return EKF_EINVAL;
+  }
+  if (ctx->scan_open) { snprintf(ctx->err, sizeof ctx->err, "ekf_insert_lines inside an open scan"); return EKF_ESTATE; }
+  NOT_POISONED(ctx);
+  CU(cudaSetDevice(ctx->cfg.device));
+  int rc = read_state(ctx);               /* the exact line count; nothing is changed before the capacity is checked */
+  if (rc) return rc;
+  const int L = ctx->h_st->L;
+  if ((long long)L + k > ctx->g.cap) {
+    snprintf(ctx->err, sizeof ctx->err, "ekf_insert_lines: %d + %d landmarks exceed the capacity of %d (nothing was inserted)", L, k, ctx->g.cap);
+    return EKF_ECAPACITY;
+  }
+  if (k == 0) { if (n_lines) *n_lines = L; return EKF_OK; }
+  rc = drain(ctx);                        /* no sweep in flight, no open group: Pbuf[rd] is the one complete covariance */
+  if (rc) return rc;
+  const int nl_old = 3 + 2 * L, nl = nl_old + 2 * k;
+  std::vector<double> hot((size_t)5 * k);
+  for (int e = 0; e < k; ++e) {
+    const size_t a = 2 * (size_t)e;
+    hot[5 * e] = lines[a]; hot[5 * e + 1] = lines[a + 1];
+    hot[5 * e + 2] = cov ? cov[a * w + a] : 0.0;
+    hot[5 * e + 3] = cov ? cov[a * w + a + 1] : 0.0;
+    hot[5 * e + 4] = cov ? cov[(a + 1) * w + a + 1] : 0.0;
+  }
+  size_t rows_per = kStageElems / w;
+  if (rows_per > w) rows_per = w;
+  rc = ensure_stage(ctx, hot.size() > rows_per * w ? hot.size() : rows_per * w);
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(ctx->d_stage, hot.data(), hot.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+  CU(ekf_launch_insert_hot(ctx->g, ctx->b, L, k, ctx->d_stage, ctx->stream));
+  const size_t ld = ctx->g.ld;
+  /* the rows above the new block: 2k zeros each (and, surveyed, the new rows too) */
+  CU(ekf_launch_insert_cold(ctx->b.P, ld, nl_old, nl, 3, (cov ? nl_old : nl) - 3, 0, 0, ctx->stream));
+  ctx->launches += 2;
+  if (cov) {
+    for (size_t i0 = 0; i0 < w; i0 += rows_per) {
+      const size_t cnt = w - i0 < rows_per ? w - i0 : rows_per;
+      CU(cudaMemcpyAsync(ctx->d_stage, cov + i0 * w, cnt * w * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+      CU(ekf_launch_insert_cold(ctx->b.P, ld, nl_old, nl, nl_old + (int)i0, (int)cnt, ctx->d_stage, (int)i0, ctx->stream));
+      CU(cudaStreamSynchronize(ctx->stream));
+      ctx->launches++;
+    }
+  }
+  ctx->h_st->L = L + k;
+  CU(cudaMemcpyAsync(&ctx->b.st->L, &ctx->h_st->L, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  ctx->L_ub = L + k;
+  ctx->snap_inflight = 0;
+  if (n_lines) *n_lines = L + k;
+  return EKF_OK;
+}
+
 /* An absolute pose fix is a rank-d (d <= 3) update whose gain needs only P[:, 0:3], which is hot storage and current at
  * all times.  The call drains first (no open sweep group, no sweep in flight: Pbuf[rd] is the one complete covariance),
  * then enqueues the gain, the hot update and one in-place sweep of (at most) two rank-2 terms.  A rejected fix or a

@@ -157,6 +157,13 @@ cudaError_t ekf_launch_remove_hot(const EkfGeom& g, const EkfBuffers& b, const i
                                   cudaStream_t s);
 cudaError_t ekf_launch_remove_cold(const double* src, size_t ld_src, int src_row0, double* dst, size_t ld_dst, int dst_row0,
                                    const int* keep, int r0, int nr, int nl, int c_from, cudaStream_t s);
+/* landmark insertion (ekf_insert_lines): k new landmarks L .. L+k-1 appended after the L live ones.
+ * hot: src = 5 doubles per new landmark (alfa, r, C[a,a], C[a,b], C[b,b]) -> y (alfa wrapped), zero `top` columns and the
+ * 2x2 diagonal blocks; cold: rows [r0, r0 + nr) of the single-GPU P (row stride ld), columns max(r, nl_old) .. nl-1: zeros
+ * for r < nl_old, else row r - nl_old of the 2k-wide new block (its row i at blk + (i - blk_row0) * 2k; blk = NULL: zeros). */
+cudaError_t ekf_launch_insert_hot(const EkfGeom& g, const EkfBuffers& b, int L, int k, const double* src, cudaStream_t s);
+cudaError_t ekf_launch_insert_cold(double* P, size_t ld, int nl_old, int nl, int r0, int nr, const double* blk, int blk_row0,
+                                   cudaStream_t s);
 /* absolute pose fix (ekf_observe_pose), d = 1..3 selected components, on the complete in-place covariance.
  * gain: S, S^-1, v, d2 and the decision (into st->fix_*), and the gain rows as two rank-2 terms: term 1
  * (K_0, K_1 ; KS_0, KS_1) into pending slot 0, term 2 (K_2, 0 ; KS_2, 0) into (K2, KS2) (slot 1, or a scratch row when

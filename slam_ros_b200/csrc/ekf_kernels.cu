@@ -1816,6 +1816,48 @@ __global__ void __launch_bounds__(EKF_BLOCK) k_remove_cold(const double* __restr
 }
 
 /* ------------------------------------------------------------------------------------------------ */
+/* Landmark insertion (ekf_insert_lines, DESIGN section 3.3): y' = [y, lines], P' = [[P, 0], [0, C]], pure data movement.
+ * The new landmarks are j = L .. L+k-1, state indices nl_old .. nl-1 (nl_old = 3 + 2 L, nl = nl_old + 2 k). */
+
+/* Hot storage.  src[5 e .. 5 e + 5) = (alfa, r, C[a,a], C[a,b], C[b,b]) of new landmark e: its y entries (alfa wrapped
+ * as the augmentation wraps it, Robot.cpp:801), its zero columns of `top` and its 2x2 diagonal block (pad 0, as
+ * k_end_scan_a writes it). */
+__global__ void __launch_bounds__(EKF_BLOCK) k_insert_hot(EkfGeom g, EkfBuffers b, int L, int k,
+                                                          const double* __restrict__ src) {
+  for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < k; e += gridDim.x * blockDim.x) {
+    const double* s = src + 5 * e;
+    const int a = 3 + 2 * (L + e);
+    double alfa = s[0];
+    normalize_radian(alfa);
+    b.y[a] = alfa; b.y[a + 1] = s[1];
+    for (int q = 0; q < 3; ++q) { b.top[(size_t)q * g.ld + a] = 0.0; b.top[(size_t)q * g.ld + a + 1] = 0.0; }
+    double* dg = b.diag + 4 * (size_t)(L + e);
+    dg[0] = s[2]; dg[1] = s[3]; dg[2] = s[4]; dg[3] = 0.0;
+  }
+}
+
+/* Cold covariance, rows [r0, r0 + nr) of the live upper triangle, columns max(r, nl_old) .. nl-1 (the new columns).  A row
+ * above the new block (r < nl_old) gets zeros; a new row gets row r - nl_old of the new block C (2k wide, row i of it at
+ * blk + (i - blk_row0) * 2k), or zeros when blk = NULL.  One CTA per row: a scalar store up to the first 16-byte boundary,
+ * then double2 streaming stores along the row (rows start on 2 KB boundaries, so even columns are 16-byte aligned). */
+__global__ void __launch_bounds__(EKF_BLOCK) k_insert_cold(double* __restrict__ P, size_t ld, int nl_old, int nl, int r0,
+                                                           int nr, const double* __restrict__ blk, int blk_row0) {
+  const int w = nl - nl_old;
+  for (int i = blockIdx.x; i < nr; i += gridDim.x) {
+    const int r = r0 + i;
+    const int c0 = max(r, nl_old);
+    double* d = P + (size_t)r * ld;
+    const double* s = (blk && r >= nl_old) ? blk + (size_t)(r - nl_old - blk_row0) * w - nl_old : 0;
+    int c = c0;
+    if (c & 1) { if (threadIdx.x == 0) __stcs(d + c, s ? __ldg(s + c) : 0.0); ++c; }
+    for (int q = c + 2 * threadIdx.x; q < nl; q += 2 * EKF_BLOCK) {
+      if (q + 1 < nl) __stcs(reinterpret_cast<double2*>(d + q), s ? make_double2(__ldg(s + q), __ldg(s + q + 1)) : make_double2(0.0, 0.0));
+      else __stcs(d + q, s ? __ldg(s + q) : 0.0);
+    }
+  }
+}
+
+/* ------------------------------------------------------------------------------------------------ */
 /* Absolute pose fix (ekf_observe_pose, DESIGN section 3.2).  H = the D selected rows of [I_3 0], so P H' is D columns of
  * P among 0..2 -- all in `top`, hot and always current -- and H P H' is a D x D block of the robot rows.  The arithmetic is
  * the reference-BLAS pattern of Robot.cpp:516-602 with D x D blocks: PHt = P H', S = H P H' + R, S^-1 by LU, d2 = v' S^-1 v
@@ -2350,6 +2392,17 @@ cudaError_t ekf_launch_remove_cold(const double* src, size_t ld_src, int src_row
   if (nr <= 0) return cudaSuccess;
   if (keep) k_remove_cold<true><<<nr, EKF_BLOCK, 0, s>>>(src, ld_src, src_row0, dst, ld_dst, dst_row0, keep, r0, nr, nl, c_from);
   else k_remove_cold<false><<<nr, EKF_BLOCK, 0, s>>>(src, ld_src, src_row0, dst, ld_dst, dst_row0, keep, r0, nr, nl, c_from);
+  return cudaGetLastError();
+}
+cudaError_t ekf_launch_insert_hot(const EkfGeom& g, const EkfBuffers& b, int L, int k, const double* src, cudaStream_t s) {
+  if (k <= 0) return cudaSuccess;
+  k_insert_hot<<<blocks_for(k, 148 * 8), EKF_BLOCK, 0, s>>>(g, b, L, k, src);
+  return cudaGetLastError();
+}
+cudaError_t ekf_launch_insert_cold(double* P, size_t ld, int nl_old, int nl, int r0, int nr, const double* blk, int blk_row0,
+                                   cudaStream_t s) {
+  if (nr <= 0 || nl <= nl_old) return cudaSuccess;
+  k_insert_cold<<<nr, EKF_BLOCK, 0, s>>>(P, ld, nl_old, nl, r0, nr, blk, blk_row0);
   return cudaGetLastError();
 }
 cudaError_t ekf_launch_pose_gain(const EkfGeom& g, const EkfBuffers& b, const EkfPoseFix& f, int d, double2* K2,

@@ -45,7 +45,7 @@ def library_path():
 SYMBOLS = [
     "ekf_default_config", "ekf_create", "ekf_destroy", "ekf_last_error", "ekf_predict", "ekf_associate",
     "ekf_update", "ekf_add_line", "ekf_end_scan", "ekf_scan", "ekf_scan_device", "ekf_sync", "ekf_get_state",
-    "ekf_get_robot_cov", "ekf_get_ellipse", "ekf_download", "ekf_upload", "ekf_remove_lines", "ekf_observe_pose",
+    "ekf_get_robot_cov", "ekf_get_ellipse", "ekf_download", "ekf_upload", "ekf_remove_lines", "ekf_insert_lines", "ekf_observe_pose",
     "ekf_download_live",
     "ekf_download_block", "ekf_cov_stats", "ekf_profile_enable", "ekf_profile_read", "ekf_profile_read_lines", "ekf_timer_start", "ekf_timer_stop", "ekf_sweep_probe",
     "ekf_nccl_unique_id", "ekf_create_sharded", "ekf_shard_ipc_handle", "ekf_shard_connect", "ekf_shard_use_fused", "ekf_batch_create", "ekf_batch_destroy", "ekf_batch_scan",
@@ -91,6 +91,7 @@ def load_library():
     lib.ekf_download.argtypes = [vp, _dp, _dp, _ip]
     lib.ekf_upload.argtypes = [vp, _dp, _dp, C.c_int]
     lib.ekf_remove_lines.argtypes = [vp, C.c_int, _ip, _ip]
+    lib.ekf_insert_lines.argtypes = [vp, C.c_int, _dp, _dp, _ip]
     lib.ekf_observe_pose.argtypes = [vp, C.c_int, _dp, _dp, C.c_double, _dp, _ip, _dp]
     lib.ekf_download_live.argtypes = [vp, _dp, _dp, C.c_int, C.c_int, _ip]
     lib.ekf_download_block.argtypes = [vp, C.c_int, C.c_int, C.c_int, C.c_int, _dp]
@@ -316,6 +317,20 @@ class EkfFilter:
         L = C.c_int(0)
         self._check(self._lib.ekf_remove_lines(self._h, idx.size, idx.ctypes.data_as(_ip) if idx.size else None,
                                                C.byref(L)), "ekf_remove_lines")
+        return int(L.value)
+
+    def insert_lines(self, lines, cov=None):
+        """Appends k known landmarks after the existing ones: lines = k x (alfa, r) in the world frame (alfa wrapped as
+        the augmentation wraps it), cov = None (surveyed: zero covariance, fixed from then on) or their 2k x 2k joint
+        covariance; zero cross-covariance with the rest.  All or nothing (EKF_ECAPACITY when they do not fit).  Returns
+        the new line count."""
+        la = _arr(lines).reshape(-1)
+        if la.size % 2:
+            raise ValueError("insert_lines: lines must be (alfa, r) pairs")
+        k = la.size // 2
+        ca = _arr(cov, (2 * k, 2 * k)) if cov is not None else None
+        L = C.c_int(0)
+        self._check(self._lib.ekf_insert_lines(self._h, k, _p(la) if k else None, _p(ca), C.byref(L)), "ekf_insert_lines")
         return int(L.value)
 
     def observe_pose(self, z, R, mask=7, d2_max=float("inf")):

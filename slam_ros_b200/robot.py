@@ -122,6 +122,13 @@ class Robot:
         Returns the new savedLineCount."""
         return self._f.remove_lines(indices)
 
+    def insert_lines(self, lines, cov=None):
+        """Not in the reference: appends known landmarks (ekf_insert_lines): lines = k x (alfa, r) in the world frame,
+        cov = None for surveyed walls (fixed from then on) or the 2k x 2k joint covariance of an earlier map.  Insert a
+        floor plan before the first localize (first fit takes the lowest index) and again after a map reset drops it.
+        Returns the new savedLineCount."""
+        return self._f.insert_lines(lines, cov)
+
     def observe_pose(self, z, R, mask=7, d2_max=float("inf")):
         """Not in the reference: fuses an absolute pose measurement (ekf_observe_pose; z = (x, y, theta), R its 3x3
         covariance, mask of EKF_POSE_X | EKF_POSE_Y | EKF_POSE_THETA).  The pose mirrors xPos / yPos / thetaPos follow
